@@ -36,6 +36,8 @@ KERNEL_NAMES = {"res2": "k_ekf_res2_step<12, 3> (two filters per warp, both Sigm
                 "fas": "k_ekf_fast_step<12, BULK> (register fragments, ekf_fast.cuh)", "pair": "k_ekf_pair_step<12> (ekf_pair.cuh)",
                 "sta": "k_ekf_static_step<12> (ekf_static.cuh)"}
 BYTES_PER_FILTER_STEP = 2 * 8 * (LEN + LEN * LEN) + 16 + 20 * N_LANDMARKS
+# filters sampled by --dump-outputs: x, Sigma, seen and status of 8192 filters come to 50 MB of float64
+DUMP_FILTERS = 8192
 METRIC = "EKF predict+update filter-steps/s (64K filters x 12 landmarks per GPU, fp64, known correspondence)"
 UNIT = "filter-steps/s"
 
@@ -200,6 +202,17 @@ def config_dict(world):
             "parallelism": f"filters sharded {world}x, no data-path collective; final NCCL all_gather of states + all_reduce of error statistics"}
 
 
+def dump_outputs(out_dir, state):
+    """--dump-outputs: the state the last timed step left (x, Sigma [row, col], seen, status, as BatchedExtendedKalman.get_state
+    returns it) for a fixed, seeded sample of DUMP_FILTERS filters, whose indices go to filters.npy; all as float64 .npy files."""
+    x, sigma, seen, status = state
+    B = x.shape[0]
+    idx = np.sort(np.random.default_rng(0).choice(B, size=min(B, DUMP_FILTERS), replace=False))
+    out_dir.mkdir(parents=True, exist_ok=True)
+    for name, a in (("filters", idx), ("x", x[idx]), ("sigma", sigma[idx]), ("seen", seen[idx]), ("status", status[idx])):
+        np.save(out_dir / f"{name}.npy", np.ascontiguousarray(a, dtype=np.float64))
+
+
 def e2e_leg(eng, torch, dist, world, dev, B, twists, zs, ids, t, K, dry, packed):
     """The same metric through the public host-buffer API: pinned host buffers, every step copies its inputs host -> device and its
     resulting state vector device -> host inside the timed region, three steps in flight.
@@ -321,6 +334,8 @@ def run_ours(args):
     if world > 1:
         dist.all_reduce(ms_t, op=dist.ReduceOp.MAX)
     ms_max = float(ms_t.item())
+    if args.dump_outputs and rank == 0:   # after the clock sampler has stopped: the copy and the writes are not part of the timed region
+        dump_outputs(Path(args.dump_outputs), eng.get_state())
     # K6: the shard's error statistics, reduced on the device (truth: the trajectory the measurements were generated from)
     from shermbot_navigation_b200 import synth
     poses = synth.true_trajectory(synth.wheel_twists(total_steps + 1, first_step_straight=True))
@@ -526,7 +541,12 @@ def main():
     ap.add_argument("--config", default="ekf", choices=["ekf", "scan", "assoc", "large", "closed_loop"],
                     help="ekf (default): the headline line of BASELINE.json configs[1] with the other configurations under `extra`; "
                          "the others run one per-config bench under tools/ on one GPU and print its own JSON line")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the state of the last one (rank 0's filters, a fixed sample of "
+                         f"{DUMP_FILTERS}) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.config != "ekf"):
+        ap.error("--dump-outputs applies to the headline run (--impl ours, --config ekf)")
     if args.config != "ekf":
         import runpy
         tool = {"scan": "bench_scan.py", "assoc": "bench_assoc.py", "large": "bench_large.py", "closed_loop": "bench_closed_loop.py"}[args.config]

@@ -4,10 +4,11 @@ CPU checker for the CUDA EKF-SLAM / circle-fit path. Two interchangeable librari
 ``oracle/oracle_api.h``:
 
 * ``load("ref")``  -> ``oracle/_ref/libnuslam_ref.so``: the UNMODIFIED reference sources
-  (``/root/reference/nuslam/src/{slam_library,circle_fit_library}.cpp`` and
-  ``/root/reference/rigid2d/src/{rigid2d,diff_drive}.cpp``) compiled where they lie against
-  ``oracle/shim/`` (Armadillo + ROS message stand-ins).  Built only in the container that has
-  ``/root/reference``; the built ``.so`` travels to the GPU box.
+  (``nuslam/src/{slam_library,circle_fit_library}.cpp`` and ``rigid2d/src/{rigid2d,diff_drive}.cpp``
+  of a checkout of sziselman/Shermbot-Navigation) compiled where they lie against
+  ``oracle/shim/`` (Armadillo + ROS message stand-ins).  Built only where such a checkout is found
+  (``reference_dir()``: ``$NUSLAM_REFERENCE``, else oracle/Makefile's default ``REF``); the reference is
+  not part of this repository.
 * ``load("port")`` -> ``oracle/libnuslam_oracle.so``: the plain-C restatement (``nuslam_oracle.c``).
 
 Only ``tests/``, ``__graft_entry__.smoke()`` and ``bench.py``'s ``cpu_baseline`` /
@@ -32,14 +33,22 @@ _fp = C.POINTER(C.c_float)
 _sp = C.POINTER(C.c_short)
 
 
+def reference_dir() -> Path | None:
+    """The checkout of the reference project that oracle/Makefile builds oracle/_ref from (its REF: $NUSLAM_REFERENCE, else the
+    Makefile's default), if it exists and can be read (os.path.isdir is False, not an error, for a path the user may not stat)."""
+    out = subprocess.run(["make", "-s", "--no-print-directory", "-C", str(HERE), "print-ref"], capture_output=True, text=True)
+    d = out.stdout.strip()
+    return Path(d) if out.returncode == 0 and d and os.path.isdir(d) else None
+
+
 def build(verbose: bool = False) -> None:
-    """Compile the C restatement and, when /root/reference is present, oracle/_ref."""
+    """Compile the C restatement and, when reference_dir() is set, oracle/_ref."""
     out = subprocess.run(["make", "-C", str(HERE), "all"], capture_output=True, text=True)
     if verbose or out.returncode != 0:
         print(out.stdout, out.stderr)
     if out.returncode != 0:
         raise RuntimeError("oracle build failed")
-    # the reference's own circle-fit test against the B200 facade (needs /root/reference and the built CUDA library; a no-op otherwise)
+    # the reference's own circle-fit test against the B200 facade (needs reference_dir() and the built CUDA library; a no-op otherwise)
     out = subprocess.run(["make", "-C", str(HERE), "facade_tests"], capture_output=True, text=True)
     if verbose or out.returncode != 0:
         print(out.stdout, out.stderr)
@@ -335,7 +344,7 @@ class TubeWorldRef:
 
     def __init__(self):
         if not self.PATH.exists():
-            raise FileNotFoundError(f"{self.PATH} missing: run oracle.build() where /root/reference is present")
+            raise FileNotFoundError(f"{self.PATH} missing: run oracle.build() where reference_dir() finds the reference")
         self._c = c = C.CDLL(str(self.PATH))
         c.twref_flavour.restype = C.c_char_p
         c.twref_lidar.argtypes = [C.c_double, C.c_double, C.c_double, _dp, C.c_double, C.c_double, _fp]

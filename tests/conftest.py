@@ -17,7 +17,7 @@ def pytest_configure(config):
 def oracle_libs():
     """Build (if needed) and load the oracle: the compiled reference when present, and the C restatement."""
     import oracle
-    if not oracle.available("port") or (Path("/root/reference").exists() and not oracle.available("ref")):
+    if not oracle.available("port") or (oracle.reference_dir() and not oracle.available("ref")):
         oracle.build()
     libs = {"port": oracle.load("port")}
     if oracle.available("ref"):

@@ -645,7 +645,7 @@ GOLDEN = __import__("pathlib").Path(__file__).resolve().parent / "golden" / "ekf
 @pytest.mark.parametrize("tag", ["known", "unknown"])
 def test_against_committed_golden_vectors(cuda_lib, mode, tag):
     """The CUDA path against tests/golden/ekf_golden.npz directly -- vectors written by tests/golden/make_golden.py from the UNMODIFIED
-    reference sources (oracle/_ref) in the container that holds /root/reference -- so that parity does not rest on the restatement
+    reference sources (oracle/_ref) built from a reference checkout -- so that parity does not rest on the restatement
     on a box without _ref. Warm start from the golden state after the first step (every first touch lies behind it), 24 free-running
     steps: association ids bit-exact, final state and covariance <= 1e-9."""
     g = np.load(GOLDEN)

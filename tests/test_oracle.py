@@ -1,17 +1,29 @@
 """CPU tests: the oracle is pinned before it is trusted.
 
 * the C restatement (oracle/nuslam_oracle.c) against the compiled, unmodified reference (oracle/_ref) --
-  bit for bit -- whenever oracle/_ref exists (it is built in the container that has /root/reference and
-  travels to the GPU box as a prebuilt .so);
+  bit for bit -- whenever oracle/_ref exists (it is built where a checkout of the reference project is
+  found: oracle.reference_dir(), oracle/Makefile REF);
 * both against the reference's own known answers: nuslam/tests/circle_tests.cpp:38-40,67-69 and
   rigid2d/tests/{tests,diff_drive_tests}.cpp;
 * both against the committed golden vectors under tests/golden/ (generated from oracle/_ref by
-  tests/golden/make_golden.py).
+  tests/golden/make_golden.py);
+* every flavour present against tests/golden/parity_golden.npz, bit for bit: the inputs and outputs of the parity tests below, so
+  that they check the restatement where the reference is absent (the file records which flavour wrote it).
 """
+from pathlib import Path
+
 import numpy as np
 import pytest
 
+from golden import make_golden as mg
 from shermbot_navigation_b200 import synth
+
+PARITY = Path(__file__).parent / "golden" / "parity_golden.npz"
+
+
+@pytest.fixture(scope="module")
+def parity():
+    return np.load(PARITY)
 
 KAT1 = np.array([[1, 7], [2, 6], [5, 8], [7, 7], [9, 5], [3, 7]], dtype=float)
 KAT2 = np.array([[-1, 0], [-0.3, -0.06], [0.3, 0.1], [1, 0]], dtype=float)
@@ -34,45 +46,29 @@ def test_circle_fit_known_answers(oracle_libs, kind):
     assert L.circle_fit(KAT2[:3])[0] == -1   # fewer than 4 points: marker.id = -1 (circle_fit_library.cpp:72-76)
 
 
-def test_port_matches_reference_ekf_bitwise(oracle_libs):
-    if "ref" not in oracle_libs:
-        pytest.skip("oracle/_ref not built here")
-    ref, port = oracle_libs["ref"], oracle_libs["port"]
-    for geometry, ids_known in (("benign", True), ("adversarial", True), ("benign", False), ("adversarial", False)):
+def test_port_matches_reference_ekf_bitwise(oracle_libs, parity):
+    """40-step batch runs, both geometries, known and unknown ids: every flavour present reproduces the stored state, status,
+    association ids and per-step trace (stored as a digest of its bytes) bit for bit (with the reference present: restatement ==
+    reference)."""
+    for geometry, ids_known in mg.EKF_VARIANTS:
         sc = synth.ekf_scenario(6, 40, geometry=geometry, seed=99)
         ids = sc["ids"] if ids_known else None
-        a = ref.ekf_run(12, sc["robot0"], sc["map0"], sc["Q"], sc["R"], sc["twists"], sc["z"], ids, trace=True)
-        b = port.ekf_run(12, sc["robot0"], sc["map0"], sc["Q"], sc["R"], sc["twists"], sc["z"], ids, trace=True)
-        for k in ("x", "sigma", "seen", "status", "ids_out", "trace"):
-            assert np.array_equal(a[k], b[k], equal_nan=True), (geometry, ids_known, k)
+        for kind, L in oracle_libs.items():
+            a = L.ekf_run(12, sc["robot0"], sc["map0"], sc["Q"], sc["R"], sc["twists"], sc["z"], ids, trace=True)
+            tag = mg.ekf_tag(geometry, ids_known)
+            for k in ("x", "sigma", "seen", "status", "ids_out"):
+                assert np.array_equal(a[k], parity[f"{tag}_{k}"], equal_nan=True), (kind, geometry, ids_known, k)
+            assert a["trace"].shape == (40, 6, 27) and mg.sha256(a["trace"]) == str(parity[f"{tag}_trace_sha256"]), (kind, geometry, ids_known)
 
 
-def test_port_matches_reference_single_calls(oracle_libs):
-    if "ref" not in oracle_libs:
-        pytest.skip("oracle/_ref not built here")
-    ref, port = oracle_libs["ref"], oracle_libs["port"]
-    sc = synth.ekf_scenario(1, 6, n=6, seed=5)
-    fa = ref.ekf(6, sc["robot0"][0], sc["map0"][0], sc["Q"], sc["R"])
-    fb = port.ekf(6, sc["robot0"][0], sc["map0"][0], sc["Q"], sc["R"])
-    for t in range(6):
-        tw = sc["twists"][t, 0]
-        fa.predict(*tw)
-        fb.predict(*tw)
-        for i in range(6):
-            z = sc["z"][t, 0, i]
-            ia, ib = fa.associate(z), fb.associate(z)
-            assert ia == ib
-            if ia > 0:
-                if t == 0:
-                    fa.init_landmark(z, ia)
-                    fb.init_landmark(z, ib)
-                assert np.array_equal(fa.zhat(ia), fb.zhat(ib))
-                assert np.array_equal(fa.H(ia), fb.H(ib))
-                fa.update(z, ia)
-                fb.update(z, ib)
-            xa, sa, na = fa.get()
-            xb, sb, nb = fb.get()
-            assert np.array_equal(xa, xb) and np.array_equal(sa, sb) and na == nb
+def test_port_matches_reference_single_calls(oracle_libs, parity):
+    """predict / associate / init_landmark / zhat / H / update one call at a time (make_golden.single_calls): every intermediate
+    output of every flavour present equals the stored one bit for bit."""
+    for kind, L in oracle_libs.items():
+        got = mg.single_calls(L)
+        for k, v in got.items():
+            assert np.array_equal(v, parity[f"calls_{k}"], equal_nan=True), (kind, k)
+        assert (got["ids"] > 0).sum() > 5   # the sequence did run updates
 
 
 def test_map_full_is_flagged(oracle_libs):
@@ -89,17 +85,19 @@ def test_map_full_is_flagged(oracle_libs):
         assert ids[0] == 1 and ids[1] == 2 and ids[2] == -1000
 
 
-def test_port_matches_reference_scans_bitwise(oracle_libs):
-    if "ref" not in oracle_libs:
-        pytest.skip("oracle/_ref not built here")
-    ref, port = oracle_libs["ref"], oracle_libs["port"]
+def test_port_matches_reference_scans_bitwise(oracle_libs, parity):
+    """1 500 scans per noise level: a fixed sample of 256 of them, detected within the full batch, equals the stored detections bit
+    for bit in every flavour present; with the reference present the two flavours also agree on the whole batch."""
     for noise in (0.0, 0.002):
-        s = synth.scan_scenario(1500, seed=31, noise_sigma=noise)
-        a = ref.scan_detect_batch(s["ranges"], s["min_range"], s["max_range"])
-        b = port.scan_detect_batch(s["ranges"], s["min_range"], s["max_range"])
-        for k in a:
-            assert np.array_equal(a[k], b[k], equal_nan=True), k
-        assert (a["n_circles"] > 0).mean() > 0.5
+        idx, s = mg.scan_sample(noise)
+        out = {kind: L.scan_detect_batch(s["ranges"], s["min_range"], s["max_range"]) for kind, L in oracle_libs.items()}
+        for kind, a in out.items():
+            for k in a:
+                assert np.array_equal(a[k][idx], parity[f"scan{noise}_{k}"], equal_nan=True), (kind, noise, k)
+            assert (a["n_circles"] > 0).mean() > 0.5
+        if len(out) == 2:
+            for k in out["ref"]:
+                assert np.array_equal(out["ref"][k], out["port"][k], equal_nan=True), k
 
 
 def test_cluster_wrap_quirk(oracle_libs):
@@ -162,25 +160,22 @@ def test_golden_vectors(oracle_libs):
         assert np.array_equal(sd["circles"], d["scan_circles"], equal_nan=True)
 
 
-def test_port_matches_reference_edge_scans(oracle_libs):
-    """Corner cases of clusterPoints (empty, UB wrap, erase-loop skip, NaN ranges, every beam a closer): the restatement and
-    the compiled reference agree bit for bit."""
-    if "ref" not in oracle_libs:
-        pytest.skip("reference build absent")
-    from shermbot_navigation_b200 import synth
+def test_port_matches_reference_edge_scans(oracle_libs, parity):
+    """Corner cases of clusterPoints (empty, UB wrap, erase-loop skip, NaN ranges, every beam a closer): every flavour present
+    reproduces the stored detections bit for bit."""
     r = synth.edge_scans()
-    a = oracle_libs["ref"].scan_detect_batch(r, 0.05, 1.0)
-    b = oracle_libs["port"].scan_detect_batch(r, 0.05, 1.0)
-    for k in ("n_clusters", "n_circles"):
-        assert np.array_equal(a[k], b[k]), k
-    assert np.array_equal(a["circles"], b["circles"], equal_nan=True)
-    # the reference returns points, not beams: the driver recovers beam indices by matching coordinates, which cannot tell
-    # NaN points apart (scan 4); everywhere else the per-beam cluster ids agree
-    ok = np.ones(len(r), dtype=bool)
-    ok[4] = False
-    assert np.array_equal(a["cluster_of_beam"][ok], b["cluster_of_beam"][ok])
-    assert a["n_circles"][1] == -2000 and a["n_clusters"][4] == 5
-    assert list(np.nonzero(b["cluster_of_beam"][4] >= 0)[0]) == [11, 13, 15, 17, 19]   # erase-loop skip keeps every second cluster
+    for kind, L in oracle_libs.items():
+        a = L.scan_detect_batch(r, 0.05, 1.0)
+        for k in ("n_clusters", "n_circles"):
+            assert np.array_equal(a[k], parity[f"edge_{k}"]), (kind, k)
+        assert np.array_equal(a["circles"], parity["edge_circles"], equal_nan=True), kind
+        # the reference returns points, not beams: its driver recovers beam indices by matching coordinates, which cannot tell
+        # NaN points apart (scan 4); everywhere else the per-beam cluster ids agree
+        ok = np.ones(len(r), dtype=bool)
+        ok[4] = kind != "ref"
+        assert np.array_equal(a["cluster_of_beam"][ok], parity["edge_cluster_of_beam"][ok]), kind
+        assert a["n_circles"][1] == -2000 and a["n_clusters"][4] == 5
+    assert list(np.nonzero(parity["edge_cluster_of_beam"][4] >= 0)[0]) == [11, 13, 15, 17, 19]   # erase-loop skip keeps every second cluster
 
 
 def test_world_step_oracle_flavours_and_geometry(oracle_libs):
@@ -210,55 +205,33 @@ def test_world_step_oracle_flavours_and_geometry(oracle_libs):
     assert (r < 1.5).sum() == 6 and set(np.nonzero(r < 1.5)[0]) == {1, 2, 3, 357, 358, 359}
 
 
-def test_world_oracle_pinned_to_the_compiled_simulator_node(oracle_libs):
+def test_world_oracle_pinned_to_the_compiled_simulator_node(oracle_libs, parity):
     """The simulator slice is PINNED: oracle/world_oracle.h (the restatement both oracle flavours -- and through them the GPU tests of
     k_world_motion / k_world_scan -- rely on) against the UNMODIFIED nuturtlesim/src/tube_world.cpp compiled with roscpp stand-ins
-    (oracle/_ref/libtube_world_ref.so, recipe oracle/Makefile `tube_world`).
+    (oracle/_ref/libtube_world_ref.so, recipe oracle/Makefile `tube_world`) when it is built, and in every case against the stored
+    outputs of tests/golden/parity_golden.npz (make_golden.world_outputs):
       * simulate_lidar_scanner (:405-471) at 400 random robot configurations around the six reference tubes: all 360 beams bit-equal
         (the +-27 degree window centred on atan2 of RELATIVE coordinates, the truncated heading offset, the fill value included);
       * main_loop (:473-544) over a 300-step drive that runs into a tube (check_collision :371-389) with wheel slip: pose, encoder
         readings and every scan bit-equal at every step (noise-free: the node seeds its generator from random_device)."""
     import oracle
-    if not oracle.TubeWorldRef.available():
-        pytest.skip("oracle/_ref/libtube_world_ref.so not built (needs /root/reference at build time)")
-    ref = oracle.TubeWorldRef()
-    from shermbot_navigation_b200 import synth
     tubes = np.ascontiguousarray(synth.TUBES[:6], dtype=np.float64)
-    rng = np.random.default_rng(5)
+    want = {k: parity[k] for k in ("lidar_poses", "lidar", "run_poses", "run_joints", "run_scans")}
+    assert (want["lidar"] < 1.5).sum(axis=1).max() > 10   # the scans did see tubes
+    before = np.concatenate([np.zeros((1, 2)), want["run_poses"][:-1, :2]])
+    assert (np.hypot(before[:, None, 0] - tubes[None, :, 0], before[:, None, 1] - tubes[None, :, 1]).min(axis=1) <= 0.0381 + 0.08).any()  # collided
     for flavour, o in oracle_libs.items():
-        # --- lidar at random configurations: world9 with the pose set, zero command, zero dt -> the step leaves the pose alone
-        worst = 0
-        for k in range(400):
-            x, y = rng.uniform(-1.2, 1.2, 2)
-            th = rng.uniform(-7.0, 7.0)
-            if np.hypot(*(tubes - [x, y]).T).min() <= 0.0381 + 1e-6:
-                continue   # inside a tube: world_step's check_collision would move the robot before the scan
-            want = ref.lidar(x, y, th, tubes, 0.0381, 1.0)
-            w = np.array([[0.16, 0.033, x, y, th, 0.0, 0.0, 0.0, 0.0]])
-            got = o.world_step(w, np.zeros(3), None, 0.0, tubes, 0.0381, 1e-9, 1.0)[0]   # robot radius ~ 0: no collision slip
-            assert np.array_equal(got.view(np.uint32), want.view(np.uint32)), (flavour, k, x, y, th)
-            worst = max(worst, int((want < 1.5).sum()))
-        assert worst > 10   # the scans did see tubes
-        # --- main_loop: drive from the origin towards tube 1, collide, slide, keep turning; slip factor 0.02
-        T = 300
-        cmd = np.zeros((T, 3))
-        cmd[:, 1] = 0.22
-        cmd[:, 0] = 0.3 * np.sin(np.arange(T) / 17.0)
-        dirn = np.arctan2(tubes[0, 1], tubes[0, 0])
-        cmd[:40, 0] = dirn / (40 * 0.02)   # turn towards tube 1 first
-        cmd[:40, 1] = 0.0
-        poses, joints, scans, dt = ref.run(cmd, 0.16, 0.033, 0.02, tubes, 0.0381, 0.08, 1.0)
-        w = np.array([[0.16, 0.033, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0]])
-        collided = False
-        for t in range(T):
-            before = w[0, 2:4].copy()
-            r = o.world_step(w, cmd[t], np.array([0.0, 0.0, 0.02, 0.02]), dt, tubes, 0.0381, 0.08, 1.0)[0]
-            assert np.array_equal(w[0, 2:5], poses[t]), (flavour, t, w[0, 2:5], poses[t])
-            assert np.array_equal(w[0, 7:9], joints[t]), (flavour, t)
-            assert np.array_equal(r.view(np.uint32), scans[t].view(np.uint32)), (flavour, t)
-            d = np.hypot(*(tubes - before).T).min()
-            collided = collided or d <= 0.0381 + 0.08
-        assert collided   # the drive did exercise check_collision
+        got = mg.world_outputs(o, tubes)
+        for k, v in want.items():
+            assert got[k].dtype == v.dtype and np.array_equal(got[k].view(np.uint8), v.view(np.uint8)), (flavour, k)
+    if oracle.TubeWorldRef.available():
+        ref = oracle.TubeWorldRef()
+        for k, (x, y, th) in enumerate(want["lidar_poses"]):
+            assert np.array_equal(ref.lidar(x, y, th, tubes, 0.0381, 1.0).view(np.uint32), want["lidar"][k].view(np.uint32)), (k, x, y, th)
+        poses, joints, scans, dt = ref.run(mg.world_drive(tubes), 0.16, 0.033, 0.02, tubes, 0.0381, 0.08, 1.0)
+        assert dt == mg.WORLD_DT
+        assert np.array_equal(poses, want["run_poses"]) and np.array_equal(joints, want["run_joints"])
+        assert np.array_equal(scans.view(np.uint32), want["run_scans"].view(np.uint32))
 
 
 def test_shim_eig_sym_fixed_point_exit_is_bit_identical(oracle_libs):
