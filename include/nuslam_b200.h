@@ -73,7 +73,7 @@ enum
      * applied in ONE rank-2m pass on the fp64 tensor pipe: one read + one write of Sigma per scan whatever m is. Selected
      * automatically when the state is too long for the on-chip kernels (n_landmarks > ~70). nuslam_ekf_step takes known or unknown correspondence
      * (associateLandmark: one thread per candidate landmark against the pass's current covariance); the single-call
-     * nuslam_ekf_associate and the fused scan step are not offered in this mode. */
+     * nuslam_ekf_associate and the fused nuslam_ekf_scan_step (per-filter marker counts) work as in the other modes. */
     NUSLAM_MODE_LARGE = 2
 };
 

@@ -35,6 +35,8 @@ struct LargeParams
     int32_t * status;
     int32_t * strict_from;   // B or null: per filter, the first measurement slot of the pass in flight that the oracle-order tail takes
                              // (k_large_strict_tail: a landmark's first touch / initializeLandmark); >= the pass's count: none
+    const int32_t * m_valid; // B or null: filter b uses only measurement slots i < m_valid[b] of the step (fused scan step; read by the
+                             // unknown-correspondence kernels, the known-id path never receives one)
     double Q[9], R[4];
 };
 
@@ -386,14 +388,16 @@ __global__ void __launch_bounds__(256) k_large_update(const LargeParams p, const
 // in-order early exit ("the first k whose distance decides") becomes an atomicMin over the keys (k << 2 | kind) of the deciding
 // candidates. k_large_assoc_finalize then turns the winner into the id of slam.cpp:291 (and into `seen`, the status bits, the id
 // slot the update kernel reads). kind: 0 = inv(psi) throws, 1 = match (d < 0.01), 2 = ambiguous (0.01 < d < 60).
+// single_call: the single associateLandmark call (kOpAssociate) with i_pass = 0 -- it associates whatever the sticky status says.
 __global__ void __launch_bounds__(128) k_large_associate(const LargeParams p, const double * __restrict__ z, int m, int i_meas, int i_pass,
                                                          const double * __restrict__ x_cur, const int32_t * __restrict__ seen,
-                                                         int32_t * __restrict__ result, double amin, double amax)
+                                                         int32_t * __restrict__ result, double amin, double amax, bool single_call)
 {
     const int b = blockIdx.y;
     const int len = p.len;
     const int sn = seen[b];
-    if (p.status[b] & (kStatusMapFull | kStatusSingular)) return;   // the reference process died on an earlier measurement
+    if (!single_call && (p.status[b] & (kStatusMapFull | kStatusSingular))) return;   // the reference process died on an earlier measurement
+    if (p.m_valid && i_meas >= p.m_valid[b]) return;                 // past this filter's measurement count
     if (p.strict_from && p.strict_from[b] <= i_pass) return;         // this filter's measurements from i_pass on: oracle-order tail
     if (sn == 0 || 3 + 2 * sn >= len) return;                        // first landmark / full map: decided without any candidate
     const double * S = p.sigma + (int64_t) b * len * len;
@@ -471,10 +475,16 @@ __global__ void __launch_bounds__(128) k_large_associate(const LargeParams p, co
 // slam.cpp:291 for every filter: the id associateLandmark returns, its side effect on `seen`, and the status bits where it throws.
 // ids_slot: B x m scratch the update kernel reads (id <= 0: no update); ids_out: B x m or null.
 __global__ void k_large_assoc_finalize(const LargeParams p, int m, int i_meas, int i_pass, int32_t * __restrict__ seen, int32_t * __restrict__ result,
-                                       int32_t * __restrict__ ids_slot, int32_t * __restrict__ ids_out)
+                                       int32_t * __restrict__ ids_slot, int32_t * __restrict__ ids_out, bool single_call)
 {
     const int b = blockIdx.x * blockDim.x + threadIdx.x;
     if (b >= p.batch) return;
+    if (p.m_valid && i_meas >= p.m_valid[b])   // no measurement in this slot (k_large_associate left `result` untouched)
+    {
+        ids_slot[(int64_t) b * m + i_meas] = 0;
+        if (ids_out) ids_out[(int64_t) b * m + i_meas] = 0;
+        return;
+    }
     if (p.strict_from && p.strict_from[b] <= i_pass)   // already handed to the oracle-order tail (it writes ids_out itself)
     {
         result[b] = 0x7fffffff;
@@ -486,7 +496,7 @@ __global__ void k_large_assoc_finalize(const LargeParams p, int m, int i_meas, i
                          // the reference there (SURVEY.md Appendix B), so this and the pass's later measurements go to k_large_strict_tail
     const int st = p.status[b];
     const int sn = seen[b];
-    if (st & (kStatusMapFull | kStatusSingular)) id = 0;
+    if (!single_call && (st & (kStatusMapFull | kStatusSingular))) id = 0;
     else if (sn == 0)
     {
         id = 1;   // :196-200
@@ -592,7 +602,8 @@ __global__ void __launch_bounds__(32) k_large_strict_tail(const LargeParams p, c
     int sn = seen ? seen[b] : p.n;
     const int snap = seen_snapshot ? seen_snapshot[b] : 0x7fffffff;   // no step protocol: never an initializeLandmark
     const int64_t mb = (int64_t) b * m + i0;
-    for (int i = sf; i < cnt; ++i)
+    const int end = p.m_valid ? min(cnt, p.m_valid[b] - i0) : cnt;   // this filter's measurements in the pass
+    for (int i = sf; i < end; ++i)
     {
         if (status & (kStatusMapFull | kStatusSingular)) break;   // the reference process has died
         const double z0 = z[2 * (mb + i)], z1 = z[2 * (mb + i) + 1];
@@ -1048,8 +1059,9 @@ inline cudaError_t launch_large_updates(LargeParams & p, const double * z, const
         for (int k = 0; k < cnt; ++k)
         {
             k_large_associate<<<dim3((unsigned) ((p.n + 127) / 128), (unsigned) p.batch), 128, 0, st>>>(p, z, m, i0 + k, k, p.x, seen, assoc->result,
-                                                                                                     assoc->amin, assoc->amax);
-            k_large_assoc_finalize<<<(unsigned) ((p.batch + 63) / 64), 64, 0, st>>>(p, m, i0 + k, k, seen, assoc->result, assoc->ids_slot, assoc->ids_out);
+                                                                                                     assoc->amin, assoc->amax, false);
+            k_large_assoc_finalize<<<(unsigned) ((p.batch + 63) / 64), 64, 0, st>>>(p, m, i0 + k, k, seen, assoc->result, assoc->ids_slot, assoc->ids_out,
+                                                                                 false);
             k_large_update<<<grid, threads, 0, st>>>(p, z + 2 * (int64_t) i0, assoc->ids_slot + i0, m, k, p.x, p.x2, seen_snapshot, seen);
             double * tmp = p.x;
             p.x = p.x2;

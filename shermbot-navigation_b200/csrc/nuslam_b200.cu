@@ -262,10 +262,13 @@ nuslam::LargeParams make_large_params(nuslam_ekf * h)
 }
 
 // LARGE-MAP mode: m measurements in delayed passes of at most kLargeMMax; `step_protocol` adds slam.cpp:295-297
-// (initializeLandmark for ids above the scan's seen snapshot, seen = max(seen, id))
-int large_updates(nuslam_ekf * h, const double * z, const int32_t * ids, int m, bool step_protocol, int32_t * ids_out = nullptr)
+// (initializeLandmark for ids above the scan's seen snapshot, seen = max(seen, id)). m_valid (B or null, unknown correspondence
+// only): filter b uses only its first m_valid[b] measurements; the passes stay planned from m, so the step needs no host read.
+int large_updates(nuslam_ekf * h, const double * z, const int32_t * ids, int m, bool step_protocol, int32_t * ids_out = nullptr,
+                  const int32_t * m_valid = nullptr)
 {
     nuslam::LargeParams p = make_large_params(h);
+    p.m_valid = m_valid;
     nuslam::LargeAssoc assoc;
     if (!ids)
     {
@@ -279,6 +282,8 @@ int large_updates(nuslam_ekf * h, const double * z, const int32_t * ids, int m, 
         assoc.amin = h->cfg.assoc_min;
         assoc.amax = h->cfg.assoc_max;
         CU(cudaMemsetAsync(assoc.result, 0x7f, sizeof(int32_t) * h->batch, h->stream));   // any value >= every key; finalize resets to INT_MAX
+        // slots no kernel writes read 0: those a filter's oracle-order tail never reaches (past its count, or after its process died)
+        if (ids_out && m > 0) CU(cudaMemsetAsync(ids_out, 0, sizeof(int32_t) * h->batch * m, h->stream));
     }
     if (step_protocol) CU(cudaMemcpyAsync(h->lg_seen_snap, h->seen, sizeof(int32_t) * h->batch, cudaMemcpyDeviceToDevice, h->stream));
     for (int i0 = 0; i0 < m; i0 += nuslam::kLargeMMax)
@@ -290,6 +295,26 @@ int large_updates(nuslam_ekf * h, const double * z, const int32_t * ids, int m, 
     }
     // x ping-pongs between the state buffer and the scratch: leave the result in the state buffer
     if (p.x != h->x) CU(cudaMemcpyAsync(h->x, p.x, sizeof(double) * (size_t) h->len * h->batch, cudaMemcpyDeviceToDevice, h->stream));
+    return NUSLAM_OK;
+}
+
+// LARGE-MAP mode, the single associateLandmark call (kOpAssociate): no update is pending, so the candidates read Sigma as it stands
+// (pass slot 0) and no oracle-order tail follows; x and Sigma are not written. z: B x 2, id_out: B, both on the device.
+int large_associate(nuslam_ekf * h, const double * z, int32_t * id_out)
+{
+    nuslam::LargeParams p = make_large_params(h);
+    p.strict_from = nullptr;
+    int rc = h->lg_ids_slot.reserve(sizeof(int32_t) * h->batch);
+    if (!rc) rc = h->lg_assoc_result.reserve(sizeof(int32_t) * h->batch);
+    if (rc) return rc;
+    int32_t * result = static_cast<int32_t *>(h->lg_assoc_result.p);
+    CU(cudaMemsetAsync(result, 0x7f, sizeof(int32_t) * h->batch, h->stream));
+    nuslam::k_large_associate<<<dim3((unsigned) ((p.n + 127) / 128), (unsigned) p.batch), 128, 0, h->stream>>>(
+        p, z, 1, 0, 0, h->x, h->seen, result, h->cfg.assoc_min, h->cfg.assoc_max, true);
+    CU(cudaGetLastError());
+    nuslam::k_large_assoc_finalize<<<(unsigned) ((p.batch + 63) / 64), 64, 0, h->stream>>>(p, 1, 0, 0, h->seen, result,
+                                                                                          static_cast<int32_t *>(h->lg_ids_slot.p), id_out, true);
+    CU(cudaGetLastError());
     return NUSLAM_OK;
 }
 
@@ -546,7 +571,6 @@ int nuslam_ekf_predict(nuslam_ekf * h, const double * twists, int mem)
 int nuslam_ekf_associate(nuslam_ekf * h, const double * z, int32_t * id_out, int mem)
 {
     if (!h || !z || !id_out) return fail(NUSLAM_ERR_INVALID, "null argument");
-    if (h->large) return fail(NUSLAM_ERR_UNSUPPORTED, "large-map mode associates inside nuslam_ekf_step (ids == NULL); the single-call form is not offered");
     if (select_device(h)) return NUSLAM_ERR_CUDA;
     nuslam::EkfParams p = make_params(h);
     p.m = 1;
@@ -560,7 +584,7 @@ int nuslam_ekf_associate(nuslam_ekf * h, const double * z, int32_t * id_out, int
     }
     else
         p.ids_out = id_out;
-    rc = launch_strict<nuslam::kOpAssociate>(h, p);
+    rc = h->large ? large_associate(h, p.z, p.ids_out) : launch_strict<nuslam::kOpAssociate>(h, p);
     if (rc) return rc;
     if (mem == NUSLAM_HOST) CU(cudaMemcpyAsync(id_out, p.ids_out, sizeof(int32_t) * h->batch, cudaMemcpyDeviceToHost, h->stream));
     return finish(h, mem);
@@ -655,12 +679,11 @@ int step_device(nuslam_ekf * h, const nuslam::EkfParams & p)
     const int m = p.m;
     if (h->large)
     {
-        if (p.m_valid) return fail(NUSLAM_ERR_UNSUPPORTED, "large-map mode takes a uniform measurement count");
         cudaError_t e = nuslam::launch_large_predict(make_large_params(h), p.twists, h->stream);
         if (e != cudaSuccess) return cuda_fail(e, "large-map predict");
         if (m > 0)
         {
-            int rc = large_updates(h, p.z, p.ids, m, /*step_protocol=*/true, p.ids_out);
+            int rc = large_updates(h, p.z, p.ids, m, /*step_protocol=*/true, p.ids_out, p.m_valid);
             if (rc) return rc;
         }
         if (p.ids && p.ids_out && m > 0) CU(cudaMemcpyAsync(p.ids_out, p.ids, sizeof(int32_t) * h->batch * m, cudaMemcpyDeviceToDevice, h->stream));
@@ -708,7 +731,6 @@ int nuslam_ekf_scan_step(nuslam_ekf * h, const double * twists, const float * ra
 {
     if (!h || !twists || !ranges) return fail(NUSLAM_ERR_INVALID, "null handle, twists or ranges");
     if (m < 1) return fail(NUSLAM_ERR_INVALID, "m < 1");
-    if (h->large) return fail(NUSLAM_ERR_UNSUPPORTED, "the fused scan step is not offered in large-map mode");
     if (select_device(h)) return NUSLAM_ERR_CUDA;
     const size_t B = (size_t) h->batch;
     nuslam::EkfParams p = make_params(h);
