@@ -73,7 +73,8 @@ enum
      * applied in ONE rank-2m pass on the fp64 tensor pipe: one read + one write of Sigma per scan whatever m is. Selected
      * automatically when the state is too long for the on-chip kernels (n_landmarks > ~70). nuslam_ekf_step takes known or unknown correspondence
      * (associateLandmark: one thread per candidate landmark against the pass's current covariance); the single-call
-     * nuslam_ekf_associate and the fused nuslam_ekf_scan_step (per-filter marker counts) work as in the other modes. */
+     * nuslam_ekf_associate and the fused nuslam_ekf_scan_step (per-filter marker counts) work as in the other modes, and so do
+     * the NUSLAM_OPT_* variants (under NUSLAM_OPT_JOSEPH the pass is a symmetric rank-4m update). */
     NUSLAM_MODE_LARGE = 2
 };
 
@@ -106,8 +107,8 @@ typedef struct
 } nuslam_ekf_config;
 
 /* Opt-in departures from the reference (SURVEY.md 8f-4), for users who want Monte-Carlo statistics that mean something; never the
- * default because parity with the reference is the contract. They run in the oracle-order kernels (any mode; the register kernel
- * and the large-map mode implement the reference's behaviour only). */
+ * default because parity with the reference is the contract. They run in the oracle-order kernels and in large-map mode (a FAST
+ * handle with options set runs the oracle-order kernels: the register kernel implements the reference's behaviour only). */
 enum
 {
     NUSLAM_OPT_WRAP_INNOVATION = 1,     /* bearing innovation wrapped to (-pi, pi] in update and associateLandmark (reference: :229-231, :272 do not) */

@@ -12,6 +12,10 @@
 // cross-check of the delayed form. Arithmetic: fp64 with FMAs; H and z_hat through the FAST kernel's short-chain helpers; parity
 // <= 1e-9 after the first touch of a landmark (the first touch itself cancels catastrophically in the reference, SURVEY.md
 // Appendix B).
+// The NUSLAM_OPT_* variants are compile-time variants of the same kernels (template arguments; options == 0 instantiates the
+// reference's kernels unchanged): PRE_MOTION_JACOBIAN in k_large_predict_pose, WRAP_INNOVATION in the update, the association and
+// the oracle-order tail, JOSEPH as a symmetric factor form of the delayed updates (large_update) and a symmetric pass
+// (k_large_rank_update_sym: Sigma <- Sigma_bar_0 - [K | A][A | K]^T, rank 4m).
 #pragma once
 #include "ekf_strict.cuh"
 #include "fastmath.cuh"
@@ -37,11 +41,16 @@ struct LargeParams
                              // (k_large_strict_tail: a landmark's first touch / initializeLandmark); >= the pass's count: none
     const int32_t * m_valid; // B or null: filter b uses only measurement slots i < m_valid[b] of the step (fused scan step; read by the
                              // unknown-correspondence kernels, the known-id path never receives one)
+    int32_t * applied;       // B: per filter, non-zero once an update of the pass in flight went into U / V (read under JOSEPH only:
+                             // the symmetric pass leaves a filter without one untouched)
+    unsigned options;        // NUSLAM_OPT_* (0 = the reference's behaviour); the kernels take the bits as template arguments
     double Q[9], R[4];
 };
 
 // predict, part 1: pose and the two Jacobian entries (predictEstimate :71-94, getA :127-148 with theta AFTER the motion
-// update), one thread per filter; b10, b20 go to the head of the P scratch.
+// update; kPreMotion, NUSLAM_OPT_PRE_MOTION_JACOBIAN: theta BEFORE it, as WarpFilter::predict), one thread per filter; b10, b20 go to
+// the head of the P scratch.
+template <bool kPreMotion>
 __global__ void k_large_predict_pose(const LargeParams p, const double * __restrict__ twists)
 {
     const int b = blockIdx.x * blockDim.x + threadIdx.x;
@@ -72,14 +81,24 @@ __global__ void k_large_predict_pose(const LargeParams p, const double * __restr
     else
     {
         const double q = div_(dx, dth);
-        double s1, c1, s3, c3;
+        double s1, c1;
         th1 = add_(theta, dth);
         sincos(th1, &s1, &c1);
         x1 = add_(x[1], add_(mul_(-q, s0), mul_(q, s1)));
         y1 = add_(x[2], sub_(mul_(q, c0), mul_(q, c1)));
-        sincos(add_(th1, dth), &s3, &c3);
-        b10 = add_(mul_(-q, c1), mul_(q, c3));
-        b20 = add_(mul_(-q, s1), mul_(q, s3));
+        if (kPreMotion)
+        {
+            // thJ = theta: cos(thJ), cos(thJ + dth) are c0, c1 (th1 = theta + dth, the same rounding as WarpFilter's add_(thJ, dth))
+            b10 = add_(mul_(-q, c0), mul_(q, c1));
+            b20 = add_(mul_(-q, s0), mul_(q, s1));
+        }
+        else
+        {
+            double s3, c3;
+            sincos(add_(th1, dth), &s3, &c3);
+            b10 = add_(mul_(-q, c1), mul_(q, c3));
+            b20 = add_(mul_(-q, s1), mul_(q, s3));
+        }
     }
     x[0] = th1;
     x[1] = x1;
@@ -130,7 +149,8 @@ __global__ void k_large_predict_cov(const LargeParams p)
 
 inline cudaError_t launch_large_predict(const LargeParams & p, const double * twists, cudaStream_t st)
 {
-    k_large_predict_pose<<<(unsigned) ((p.batch + 63) / 64), 64, 0, st>>>(p, twists);
+    if (p.options & kOptPreMotionJacobian) k_large_predict_pose<true><<<(unsigned) ((p.batch + 63) / 64), 64, 0, st>>>(p, twists);
+    else k_large_predict_pose<false><<<(unsigned) ((p.batch + 63) / 64), 64, 0, st>>>(p, twists);
     k_large_predict_cov<<<dim3((p.len + 255) / 256, (unsigned) p.batch), 256, 0, st>>>(p);
     return cudaGetLastError();
 }
@@ -209,6 +229,15 @@ struct LargePre
     const double * z;     // [cnt][2]
 };
 
+//
+// JOSEPH (NUSLAM_OPT_JOSEPH): every update ends in the symmetric part of (I - K H) Sigma (I - K H)^T + K R K^T. With P = Sigma H^T,
+// W = H Sigma, S = H Sigma H^T + R and the symmetric parts Sigma_bar, P_bar = (P + W^T) / 2, S_bar, that is, for any K,
+//     Sigma_bar - K A^T - A K^T,   A = P_bar - K S_bar / 2,
+// so the pass stays one low-rank update: V holds A_u instead of W_u (U keeps K_u) and every consumer forms
+//     Sigma_i = Sigma_bar_0 - sum_{u<i} (K_u A_u^T + A_u K_u^T),
+// symmetric by construction (row and column of an index are one value, P = W^T, P_bar = P); the pass is k_large_rank_update_sym.
+// WRAP (NUSLAM_OPT_WRAP_INNOVATION): the bearing innovation is wrapped with normalize_angle, as in WarpFilter::update.
+template <unsigned OPT>
 __device__ __forceinline__ void large_update(const LargeParams & p, const double * __restrict__ z, const int32_t * __restrict__ ids, int m, int i,
                                              const double * __restrict__ x_old, double * __restrict__ x_new,
                                              const int32_t * __restrict__ seen_snapshot, int32_t * __restrict__ seen, double * own = nullptr,
@@ -216,7 +245,8 @@ __device__ __forceinline__ void large_update(const LargeParams & p, const double
 {
     // own (cooperative single-launch pass only): this block's shared-memory copy of ITS threads' entries of the pass's K_u / W_u,
     // own[(2 r + {0: W, 1: K}) * blockDim.x + threadIdx.x] -- the correction loop then reads no global memory at all; the global U / V
-    // rows are still written (the other blocks read five entries of them, the rank update all of them)
+    // rows are still written (the other blocks read five entries of them, the rank update all of them). JOSEPH: A_u in place of W_u.
+    constexpr bool kJoseph = (OPT & kOptJoseph) != 0, kWrap = (OPT & kOptWrapInnovation) != 0;
     const int b = blockIdx.y;
     const int len = p.len;
     const int j = blockIdx.x * blockDim.x + threadIdx.x;
@@ -268,6 +298,12 @@ __device__ __forceinline__ void large_update(const LargeParams & p, const double
             col[q] = S[j + (int64_t) idx[q] * len];
         }
     }
+    if (kJoseph && (pre || j < len))
+    {
+        // Sigma_bar_0: row and column of each index are one value from here on (col is not read again)
+#pragma unroll
+        for (int q = 0; q < 5; ++q) row[q] = 0.5 * (row[q] + col[q]);
+    }
     double xl[5];
     const bool init = large_local_state(x, c, id, z2, seen_snapshot, b, xl);
     const double x_own = (j < len) ? x[j] : 0.0;
@@ -285,13 +321,33 @@ __device__ __forceinline__ void large_update(const LargeParams & p, const double
         blk[r][q] = pre ? pre->blk[25 * i + threadIdx.x] : S[idx[r] + (int64_t) idx[q] * len];
     }
     __syncthreads();
-    if (threadIdx.x < 25)
+    if constexpr (!kJoseph)
     {
-        // Sigma_i(idx[r], idx[q]): what the owner of column idx[q] computes as row[r] below, term for term
+        if (threadIdx.x < 25)
+        {
+            // Sigma_i(idx[r], idx[q]): what the owner of column idx[q] computes as row[r] below, term for term
+            const int r = threadIdx.x / 5, q = threadIdx.x % 5;
+            double v = blk[r][q];
+            for (int u = 0; u < 2 * i; ++u) v = fma(-ku[u][r], wu[u][q], v);
+            blk[r][q] = v;
+        }
+    }
+    else
+    {
+        // the same under JOSEPH: Sigma_bar_0 (read before any thread writes), then K_u A_u^T + A_u K_u^T (wu holds A_u)
         const int r = threadIdx.x / 5, q = threadIdx.x % 5;
-        double v = blk[r][q];
-        for (int u = 0; u < 2 * i; ++u) v = fma(-ku[u][r], wu[u][q], v);
-        blk[r][q] = v;
+        double v = 0.0;
+        if (threadIdx.x < 25) v = 0.5 * (blk[r][q] + blk[q][r]);
+        __syncthreads();
+        if (threadIdx.x < 25)
+        {
+            for (int u = 0; u < 2 * i; ++u)
+            {
+                v = fma(-ku[u][r], wu[u][q], v);
+                v = fma(-wu[u][r], ku[u][q], v);
+            }
+            blk[r][q] = v;
+        }
     }
     __syncthreads();
     const LargeModel mdl = large_model(xl);
@@ -323,16 +379,35 @@ __device__ __forceinline__ void large_update(const LargeParams & p, const double
     if (j >= len) return;
     const double xj = (init && j == c) ? xl[3] : (init && j == c + 1) ? xl[4] : x_own;   // x after initializeLandmark
     if (j == 0 && seen && id > seen[b]) seen[b] = id;                                      // what associateLandmark would have done to `seen`
-#pragma unroll 4
-    for (int r = 0; r < 2 * i; ++r)
+    if constexpr (!kJoseph)
     {
-        const double wj = own ? own[(2 * r) * blockDim.x + threadIdx.x] : V[(int64_t) r * len + j];
-        const double kj = own ? own[(2 * r + 1) * blockDim.x + threadIdx.x] : U[(int64_t) r * len + j];
-#pragma unroll
-        for (int q = 0; q < 5; ++q)
+#pragma unroll 4
+        for (int r = 0; r < 2 * i; ++r)
         {
-            row[q] = fma(-ku[r][q], wj, row[q]);
-            col[q] = fma(-kj, wu[r][q], col[q]);
+            const double wj = own ? own[(2 * r) * blockDim.x + threadIdx.x] : V[(int64_t) r * len + j];
+            const double kj = own ? own[(2 * r + 1) * blockDim.x + threadIdx.x] : U[(int64_t) r * len + j];
+#pragma unroll
+            for (int q = 0; q < 5; ++q)
+            {
+                row[q] = fma(-ku[r][q], wj, row[q]);
+                col[q] = fma(-kj, wu[r][q], col[q]);
+            }
+        }
+    }
+    else
+    {
+        // twice the shared-memory operands per update of the loop above: unrolled by 2 (by 4, ptxas spills k_large_update<JOSEPH>)
+#pragma unroll 2
+        for (int r = 0; r < 2 * i; ++r)
+        {
+            const double aj = own ? own[(2 * r) * blockDim.x + threadIdx.x] : V[(int64_t) r * len + j];   // A_r(j)
+            const double kj = own ? own[(2 * r + 1) * blockDim.x + threadIdx.x] : U[(int64_t) r * len + j];
+#pragma unroll
+            for (int q = 0; q < 5; ++q)
+            {
+                row[q] = fma(-ku[r][q], aj, row[q]);
+                row[q] = fma(-wu[r][q], kj, row[q]);
+            }
         }
     }
     double pj[2];
@@ -344,11 +419,15 @@ __device__ __forceinline__ void large_update(const LargeParams & p, const double
         for (int q = 0; q < 5; ++q)
         {
             w = fma(mdl.h[a][q], row[q], w);
-            pp = fma(col[q], mdl.h[a][q], pp);
+            if (!kJoseph) pp = fma(col[q], mdl.h[a][q], pp);
         }
-        V[(int64_t) (2 * i + a) * len + j] = w;
-        if (own) own[(2 * (2 * i + a)) * blockDim.x + threadIdx.x] = w;
-        pj[a] = pp;
+        if constexpr (!kJoseph)
+        {
+            V[(int64_t) (2 * i + a) * len + j] = w;
+            if (own) own[(2 * (2 * i + a)) * blockDim.x + threadIdx.x] = w;
+            pj[a] = pp;
+        }
+        else pj[a] = w;   // P = W^T: the formed Sigma_i is symmetric
     }
     const double det = s[0][0] * s[1][1] - s[0][1] * s[1][0];
     if (det == 0.0)
@@ -356,6 +435,13 @@ __device__ __forceinline__ void large_update(const LargeParams & p, const double
         U[(int64_t) (2 * i) * len + j] = 0.0;
         U[(int64_t) (2 * i + 1) * len + j] = 0.0;
         if (own) own[(2 * (2 * i) + 1) * blockDim.x + threadIdx.x] = own[(2 * (2 * i + 1) + 1) * blockDim.x + threadIdx.x] = 0.0;
+        if constexpr (kJoseph)
+        {
+            // the pass reads both factors in both roles: both are zero
+            V[(int64_t) (2 * i) * len + j] = 0.0;
+            V[(int64_t) (2 * i + 1) * len + j] = 0.0;
+            if (own) own[(2 * (2 * i)) * blockDim.x + threadIdx.x] = own[(2 * (2 * i + 1)) * blockDim.x + threadIdx.x] = 0.0;
+        }
         xo[j] = xj;
         if (j == 0) p.status[b] |= kStatusSingular;
         return;
@@ -369,17 +455,35 @@ __device__ __forceinline__ void large_update(const LargeParams & p, const double
         own[(2 * (2 * i) + 1) * blockDim.x + threadIdx.x] = k0;
         own[(2 * (2 * i + 1) + 1) * blockDim.x + threadIdx.x] = k1;
     }
-    const double dz0 = z2[0] - mdl.zr, dz1 = z2[1] - mdl.zb;   // :272, no wrap
+    if constexpr (kJoseph)
+    {
+        // A(j, :) = P_bar(j, :) - K(j, :) S_bar / 2
+        const double sb01 = 0.5 * (s[0][1] + s[1][0]);
+        const double a0 = pj[0] - 0.5 * (k0 * s[0][0] + k1 * sb01);
+        const double a1 = pj[1] - 0.5 * (k0 * sb01 + k1 * s[1][1]);
+        V[(int64_t) (2 * i) * len + j] = a0;
+        V[(int64_t) (2 * i + 1) * len + j] = a1;
+        if (own)
+        {
+            own[(2 * (2 * i)) * blockDim.x + threadIdx.x] = a0;
+            own[(2 * (2 * i + 1)) * blockDim.x + threadIdx.x] = a1;
+        }
+        if (j == 0) p.applied[b] = 1;
+    }
+    double dz1 = z2[1] - mdl.zb;   // :272, no wrap unless opted in
+    if (kWrap) dz1 = normalize_angle(dz1);
+    const double dz0 = z2[0] - mdl.zr;
     double xn = xj + (k0 * dz0 + k1 * dz1);
     if (j == 0) xn = wrap_angle(xn);   // normalize_angle, slam_library.cpp:276
     xo[j] = xn;
 }
 
+template <unsigned OPT>
 __global__ void __launch_bounds__(256) k_large_update(const LargeParams p, const double * __restrict__ z, const int32_t * __restrict__ ids, int m, int i,
                                                       const double * __restrict__ x_old, double * __restrict__ x_new,
                                                       const int32_t * __restrict__ seen_snapshot, int32_t * __restrict__ seen)
 {
-    large_update(p, z, ids, m, i, x_old, x_new, seen_snapshot, seen);
+    large_update<OPT>(p, z, ids, m, i, x_old, x_new, seen_snapshot, seen);
 }
 
 // ---- associateLandmark (slam_library.cpp:188-253) against the CURRENT covariance of a delayed pass ----
@@ -389,6 +493,8 @@ __global__ void __launch_bounds__(256) k_large_update(const LargeParams p, const
 // candidates. k_large_assoc_finalize then turns the winner into the id of slam.cpp:291 (and into `seen`, the status bits, the id
 // slot the update kernel reads). kind: 0 = inv(psi) throws, 1 = match (d < 0.01), 2 = ambiguous (0.01 < d < 60).
 // single_call: the single associateLandmark call (kOpAssociate) with i_pass = 0 -- it associates whatever the sticky status says.
+// OPT: JOSEPH forms the sub-block as large_update does under it, WRAP wraps the bearing innovation (WarpFilter::mahalanobis).
+template <unsigned OPT>
 __global__ void __launch_bounds__(128) k_large_associate(const LargeParams p, const double * __restrict__ z, int m, int i_meas, int i_pass,
                                                          const double * __restrict__ x_cur, const int32_t * __restrict__ seen,
                                                          int32_t * __restrict__ result, double amin, double amax, bool single_call)
@@ -416,21 +522,33 @@ __global__ void __launch_bounds__(128) k_large_associate(const LargeParams p, co
     if (k > sn) return;
     const int c = 3 + 2 * (k - 1);
     const int idx[5] = {0, 1, 2, c, c + 1};
+    constexpr bool kJoseph = (OPT & kOptJoseph) != 0;
     double B5[5][5];
 #pragma unroll
     for (int r = 0; r < 5; ++r)
 #pragma unroll
         for (int q = 0; q < 5; ++q) B5[r][q] = S[idx[r] + (int64_t) idx[q] * len];
+    if (kJoseph)
+    {
+#pragma unroll
+        for (int r = 0; r < 5; ++r)
+#pragma unroll
+            for (int q = r + 1; q < 5; ++q) B5[r][q] = B5[q][r] = 0.5 * (B5[r][q] + B5[q][r]);   // Sigma_bar_0
+    }
     for (int u = 0; u < 2 * i_pass; ++u)
     {
         const double kc = U[(int64_t) u * len + c], kc1 = U[(int64_t) u * len + c + 1];
         const double wc = V[(int64_t) u * len + c], wc1 = V[(int64_t) u * len + c + 1];
         const double kr[5] = {ku3[u][0], ku3[u][1], ku3[u][2], kc, kc1};
-        const double wq[5] = {wu3[u][0], wu3[u][1], wu3[u][2], wc, wc1};
+        const double wq[5] = {wu3[u][0], wu3[u][1], wu3[u][2], wc, wc1};   // JOSEPH: A_u
 #pragma unroll
         for (int r = 0; r < 5; ++r)
 #pragma unroll
-            for (int q = 0; q < 5; ++q) B5[r][q] = fma(-kr[r], wq[q], B5[r][q]);
+            for (int q = 0; q < 5; ++q)
+            {
+                B5[r][q] = fma(-kr[r], wq[q], B5[r][q]);
+                if (kJoseph) B5[r][q] = fma(-wq[r], kr[q], B5[r][q]);
+            }
     }
     const double xl[5] = {x[0], x[1], x[2], x[c], x[c + 1]};
     const LargeModel mdl = large_model(xl);
@@ -463,7 +581,9 @@ __global__ void __launch_bounds__(128) k_large_associate(const LargeParams p, co
     else
     {
         const double i00 = psi[1][1] / det, i01 = -psi[0][1] / det, i10 = -psi[1][0] / det, i11 = psi[0][0] / det;
-        const double dz0 = z0 - mdl.zr, dz1 = z1 - mdl.zb;   // no angle wrap (:229-231)
+        const double dz0 = z0 - mdl.zr;
+        double dz1 = z1 - mdl.zb;   // no angle wrap (:229-231) unless opted in
+        if (OPT & kOptWrapInnovation) dz1 = normalize_angle(dz1);
         const double t0 = dz0 * i00 + dz1 * i10, t1 = dz0 * i01 + dz1 * i11;
         const double d = t0 * dz0 + t1 * dz1;
         if (d < amin) kind = 1;
@@ -578,7 +698,8 @@ __global__ void k_large_first_touch(const LargeParams p, const int32_t * __restr
 // ekf_strict.cuh (WarpFilter working directly on the filter's Sigma in HBM; its 14 len doubles of scratch are the pass's U rows, free
 // once the rank update has run) -- associateLandmark / initializeLandmark / update exactly as EKFSlam::main_loop orders them
 // (slam.cpp:279-319). It exists for parity (a first touch costs one warp a full sweep over Sigma: ~30 ms at 4096 landmarks), the
-// steady state of a built map never takes it.
+// steady state of a built map never takes it. OPT: the NUSLAM_OPT_* bits of the handle, as in the STRICT kernels.
+template <unsigned OPT>
 __global__ void __launch_bounds__(32) k_large_strict_tail(const LargeParams p, const double * __restrict__ z, const int32_t * __restrict__ ids, int m, int i0,
                                                           int cnt, double * __restrict__ x_cur, const int32_t * __restrict__ seen_snapshot,
                                                           int32_t * __restrict__ seen, double amin, double amax, int32_t * __restrict__ ids_out)
@@ -590,7 +711,7 @@ __global__ void __launch_bounds__(32) k_large_strict_tail(const LargeParams p, c
     f.len = p.len;
     f.n = p.n;
     f.lane = lane;
-    f.opt = 0u;
+    f.opt = OPT;
     f.S = p.sigma + (int64_t) b * p.len * p.len;
     f.x = x_cur + (int64_t) b * p.len;
     double * scratch = p.U + (int64_t) b * 2 * kLargeMMax * p.len;
@@ -644,6 +765,7 @@ __global__ void __launch_bounds__(32) k_large_strict_tail(const LargeParams p, c
 
 // all `cnt` delayed updates of a pass in ONE cooperative launch: consecutive updates are separated by a grid barrier (~2 us) instead
 // of a kernel boundary (~12 us of dependent-launch latency). x ping-pongs between p.x and p.x2.
+template <unsigned OPT>
 __global__ void __launch_bounds__(64) k_large_updates_coop(const LargeParams p, const double * __restrict__ z, const int32_t * __restrict__ ids, int m, int cnt,
                                                           const int32_t * __restrict__ seen_snapshot, int32_t * __restrict__ seen)
 {
@@ -697,7 +819,7 @@ __global__ void __launch_bounds__(64) k_large_updates_coop(const LargeParams p, 
     const LargePre pre = {pre_rc, pre_blk, pre_id, pre_z};
     for (int k = 0; k < cnt; ++k)
     {
-        large_update(p, z, ids, m, k, xc, xn, seen_snapshot, seen, own, &pre);
+        large_update<OPT>(p, z, ids, m, k, xc, xn, seen_snapshot, seen, own, &pre);
         grid.sync();
         const double * t = xc;
         xc = xn;
@@ -1001,6 +1123,106 @@ inline cudaError_t launch_large_rank_update(const LargeParams & p, int kk, cudaS
     return cudaGetLastError();
 }
 
+// The JOSEPH pass: Sigma <- Sigma_bar_0 - [K | A] [A | K]^T (rank 2 kk: U holds K_u, V holds A_u, large_update), exactly symmetric.
+// The DMMA sums of (r, c) and (c, r) would run in different orders, so one CTA owns a tile PAIR (I <= J): it stages the partner tile
+// (J, I) in shared memory, starts the accumulators of tile (I, J) at (T_IJ + T_JI^T) / 2, runs the DMMAs on (I, J) only and stores
+// the tile and its transpose (a diagonal tile: its lower triangle, mirrored). Same bytes read and written as the plain pass, the
+// DMMAs of a rank-kk pass over all tiles. The operands come in fragment layout straight from L2 / L1 (as in the pipelined kernel),
+// so the rank is not bounded by a shared-memory staging area: kk up to 2 kLargeMMax, rank 4 kLargeMMax.
+// A filter with no update of the pass in its factors (frozen, or every slot handed to the oracle-order tail) is not touched at all:
+// its Sigma leaves the pass bit for bit as it came in, symmetric or not.
+constexpr int kSymLd = kLargeTile + 1;
+__global__ void __launch_bounds__(128, 4) k_large_rank_update_sym(const LargeParams p, int kk)
+{
+    __shared__ double tr[kLargeTile][kSymLd];   // tr[rr][cc] = Sigma(c0 + cc, r0 + rr): tile (J, I) transposed, then the result for it
+    const int b = blockIdx.y;
+    if (!p.applied[b]) return;
+    const int len = p.len;
+    // pair index -> (I, J), I <= J: pair = J (J + 1) / 2 + I
+    const int pair = (int) blockIdx.x;
+    int J = (int) ((sqrt(8.0 * pair + 1.0) - 1.0) * 0.5);
+    while ((J + 1) * (J + 2) / 2 <= pair) ++J;
+    while (J * (J + 1) / 2 > pair) --J;
+    const int I = pair - J * (J + 1) / 2;
+    const bool diag = I == J;
+    const int r0 = I * kLargeTile, c0 = J * kLargeTile;
+    double * S = p.sigma + (int64_t) b * len * len;
+    const double * U = p.U + (int64_t) b * 2 * kLargeMMax * len;
+    const double * V = p.V + (int64_t) b * 2 * kLargeMMax * len;
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int g = lane >> 2, t = lane & 3;
+    const int lr = 32 * (warp >> 1), lc = 32 * (warp & 1);
+    double C[4][4][2];
+#pragma unroll
+    for (int br = 0; br < 4; ++br)
+#pragma unroll
+        for (int bc = 0; bc < 4; ++bc)
+#pragma unroll
+            for (int e = 0; e < 2; ++e)
+            {
+                const int row = r0 + lr + 8 * br + g, col = c0 + lc + 8 * bc + 2 * t + e;
+                C[br][bc][e] = (row < len && col < len) ? __ldcs(S + (int64_t) col * len + row) : 0.0;
+            }
+#pragma unroll 4
+    for (int e = threadIdx.x; e < kLargeTile * kLargeTile; e += blockDim.x)
+    {
+        const int cc = e % kLargeTile, rr = e / kLargeTile;   // column r0 + rr of Sigma, rows c0 + cc: contiguous in cc
+        tr[rr][cc] = (c0 + cc < len && r0 + rr < len) ? __ldcs(S + (int64_t) (r0 + rr) * len + c0 + cc) : 0.0;
+    }
+    __syncthreads();
+#pragma unroll
+    for (int br = 0; br < 4; ++br)
+#pragma unroll
+        for (int bc = 0; bc < 4; ++bc)
+#pragma unroll
+            for (int e = 0; e < 2; ++e) C[br][bc][e] = 0.5 * (C[br][bc][e] + tr[lr + 8 * br + g][lc + 8 * bc + 2 * t + e]);
+    __syncthreads();   // tr is reused for the transposed store
+    // a = -[K | A](row, k), b = [A | K](k, column); kk is a multiple of 4, so a k-step lies in one half
+    for (int k0 = 0; k0 < 2 * kk; k0 += 4)
+    {
+        const bool second = k0 >= kk;
+        const int k = (second ? k0 - kk : k0) + t;
+        const double * Ak = (second ? V : U) + (int64_t) k * len + r0 + lr + g;
+        const double * Bk = (second ? U : V) + (int64_t) k * len + c0 + lc + g;
+        double a[4], bb[4];
+#pragma unroll
+        for (int q = 0; q < 4; ++q)
+        {
+            a[q] = (r0 + lr + 8 * q + g < len) ? -__ldg(Ak + 8 * q) : 0.0;
+            bb[q] = (c0 + lc + 8 * q + g < len) ? __ldg(Bk + 8 * q) : 0.0;
+        }
+#pragma unroll
+        for (int br = 0; br < 4; ++br)
+#pragma unroll
+            for (int bc = 0; bc < 4; ++bc) dmma884_large(C[br][bc][0], C[br][bc][1], a[br], bb[bc]);
+    }
+#pragma unroll
+    for (int br = 0; br < 4; ++br)
+#pragma unroll
+        for (int bc = 0; bc < 4; ++bc)
+#pragma unroll
+            for (int e = 0; e < 2; ++e)
+            {
+                const int rl = lr + 8 * br + g, cl = lc + 8 * bc + 2 * t + e;
+                if (r0 + rl < len && c0 + cl < len && (!diag || rl >= cl)) __stcs(S + (int64_t) (c0 + cl) * len + r0 + rl, C[br][bc][e]);
+                tr[rl][cl] = C[br][bc][e];
+            }
+    __syncthreads();
+#pragma unroll 4
+    for (int e = threadIdx.x; e < kLargeTile * kLargeTile; e += blockDim.x)
+    {
+        const int cc = e % kLargeTile, rr = e / kLargeTile;   // Sigma(c0 + cc, r0 + rr) = C(rr, cc)
+        if (c0 + cc < len && r0 + rr < len && (!diag || rr > cc)) __stcs(S + (int64_t) (r0 + rr) * len + c0 + cc, tr[rr][cc]);
+    }
+}
+
+inline cudaError_t launch_large_rank_update_sym(const LargeParams & p, int kk, cudaStream_t st)
+{
+    const unsigned tiles = (p.len + kLargeTile - 1) / kLargeTile;
+    k_large_rank_update_sym<<<dim3(tiles * (tiles + 1) / 2, (unsigned) p.batch), 128, 0, st>>>(p, kk);
+    return cudaGetLastError();
+}
+
 // initializeLandmark (slam_library.cpp:255-261) for measurement i of the step when its id exceeds the scan's seen snapshot
 // (slam.cpp:295-297), or unconditionally (snapshot == nullptr: the single initializeLandmark call); one thread per filter.
 __global__ void k_large_init_landmark(const LargeParams p, const double * __restrict__ z, const int32_t * __restrict__ ids, int m, int i,
@@ -1039,35 +1261,68 @@ struct LargeAssoc
     double amin = 0.01, amax = 60.0;
 };
 
-inline cudaError_t launch_large_updates(LargeParams & p, const double * z, const int32_t * ids, int m, int i0, int cnt,
-                                        const int32_t * seen_snapshot, int32_t * seen, cudaStream_t st, const LargeAssoc * assoc = nullptr)
+// k_large_associate for measurement i_meas of the step (slot i_pass of the pass), one thread per candidate landmark
+template <unsigned OPT>
+inline void launch_large_associate_t(const LargeParams & p, const double * z, int m, int i_meas, int i_pass, const double * x_cur, const int32_t * seen,
+                                     int32_t * result, double amin, double amax, bool single_call, cudaStream_t st)
 {
+    k_large_associate<OPT><<<dim3((unsigned) ((p.n + 127) / 128), (unsigned) p.batch), 128, 0, st>>>(p, z, m, i_meas, i_pass, x_cur, seen, result, amin,
+                                                                                                   amax, single_call);
+}
+
+// the option bits the pass kernels take as template arguments (PRE_MOTION_JACOBIAN is predict's alone)
+constexpr unsigned kLargePassOpts = kOptWrapInnovation | kOptJoseph;
+
+inline void launch_large_associate(const LargeParams & p, const double * z, int m, int i_meas, int i_pass, const double * x_cur, const int32_t * seen,
+                                   int32_t * result, double amin, double amax, bool single_call, cudaStream_t st)
+{
+    switch (p.options & kLargePassOpts)
+    {
+    case 0u: launch_large_associate_t<0u>(p, z, m, i_meas, i_pass, x_cur, seen, result, amin, amax, single_call, st); break;
+    case kOptWrapInnovation:
+        launch_large_associate_t<kOptWrapInnovation>(p, z, m, i_meas, i_pass, x_cur, seen, result, amin, amax, single_call, st);
+        break;
+    case kOptJoseph: launch_large_associate_t<kOptJoseph>(p, z, m, i_meas, i_pass, x_cur, seen, result, amin, amax, single_call, st); break;
+    default: launch_large_associate_t<kLargePassOpts>(p, z, m, i_meas, i_pass, x_cur, seen, result, amin, amax, single_call, st); break;
+    }
+}
+
+// OPT: the handle's option bits within kLargePassOpts (every static below is per instantiation: each kernel variant has its own occupancy)
+template <unsigned OPT>
+inline cudaError_t launch_large_updates_t(LargeParams & p, const double * z, const int32_t * ids, int m, int i0, int cnt,
+                                          const int32_t * seen_snapshot, int32_t * seen, cudaStream_t st, const LargeAssoc * assoc)
+{
+    constexpr bool kJoseph = (OPT & kOptJoseph) != 0;
     const int threads = 64;   // ~130 small blocks at len 8195: every SM takes part in the latency-bound row / column gathers
     const dim3 grid((p.len + threads - 1) / threads, (unsigned) p.batch);
     const int kk = (2 * cnt + 3) & ~3;
     k_large_clear_w<<<dim3((unsigned) (((int64_t) kk * p.len + threads - 1) / threads), (unsigned) p.batch), threads, 0, st>>>(p, kk / 2);
+    if (kJoseph)
+    {
+        const cudaError_t ce = cudaMemsetAsync(p.applied, 0, sizeof(int32_t) * p.batch, st);
+        if (ce != cudaSuccess) return ce;
+    }
     if (p.strict_from) k_large_first_touch<<<(unsigned) ((p.batch + 63) / 64), 64, 0, st>>>(p, ids, m, i0, cnt, seen_snapshot);
     // after the pass: measurements the delayed path left to the oracle-order tail (first touches; usually none)
     auto tail = [&]() {
         if (p.strict_from)
-            k_large_strict_tail<<<(unsigned) p.batch, 32, 0, st>>>(p, z, ids, m, i0, cnt, p.x, seen_snapshot, seen, assoc ? assoc->amin : 0.0,
-                                                                assoc ? assoc->amax : 0.0, assoc ? assoc->ids_out : nullptr);
+            k_large_strict_tail<OPT><<<(unsigned) p.batch, 32, 0, st>>>(p, z, ids, m, i0, cnt, p.x, seen_snapshot, seen, assoc ? assoc->amin : 0.0,
+                                                                     assoc ? assoc->amax : 0.0, assoc ? assoc->ids_out : nullptr);
     };
     if (assoc)
     {
         // unknown correspondence: per measurement associate (one thread per candidate) -> finalize -> update
         for (int k = 0; k < cnt; ++k)
         {
-            k_large_associate<<<dim3((unsigned) ((p.n + 127) / 128), (unsigned) p.batch), 128, 0, st>>>(p, z, m, i0 + k, k, p.x, seen, assoc->result,
-                                                                                                     assoc->amin, assoc->amax, false);
+            launch_large_associate_t<OPT>(p, z, m, i0 + k, k, p.x, seen, assoc->result, assoc->amin, assoc->amax, false, st);
             k_large_assoc_finalize<<<(unsigned) ((p.batch + 63) / 64), 64, 0, st>>>(p, m, i0 + k, k, seen, assoc->result, assoc->ids_slot, assoc->ids_out,
                                                                                  false);
-            k_large_update<<<grid, threads, 0, st>>>(p, z + 2 * (int64_t) i0, assoc->ids_slot + i0, m, k, p.x, p.x2, seen_snapshot, seen);
+            k_large_update<OPT><<<grid, threads, 0, st>>>(p, z + 2 * (int64_t) i0, assoc->ids_slot + i0, m, k, p.x, p.x2, seen_snapshot, seen);
             double * tmp = p.x;
             p.x = p.x2;
             p.x2 = tmp;
         }
-        const cudaError_t re = launch_large_rank_update(p, kk, st);
+        const cudaError_t re = kJoseph ? launch_large_rank_update_sym(p, kk, st) : launch_large_rank_update(p, kk, st);
         if (re != cudaSuccess) return re;
         tail();
         return cudaGetLastError();
@@ -1086,8 +1341,8 @@ inline cudaError_t launch_large_updates(LargeParams & p, const double * z, const
         cudaDeviceGetAttribute(&can, cudaDevAttrCooperativeLaunch, dev);
         cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
         const size_t dyn_max = ((size_t) (6 + 4 * kLargeMMax) * 64 + 25 * kLargeMMax) * sizeof(double);
-        if (cudaFuncSetAttribute(k_large_updates_coop, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) dyn_max) != cudaSuccess) can = 0;
-        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_large_updates_coop, threads, dyn_max);
+        if (cudaFuncSetAttribute(k_large_updates_coop<OPT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) dyn_max) != cudaSuccess) can = 0;
+        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_large_updates_coop<OPT>, threads, dyn_max);
         coop_blocks_per_sm = can ? nb * sms : 0;
     }
     if ((int64_t) grid.x * grid.y <= coop_blocks_per_sm)
@@ -1096,7 +1351,7 @@ inline cudaError_t launch_large_updates(LargeParams & p, const double * z, const
         const int32_t * ii = ids + i0;
         void * args[] = {(void *) &p, (void *) &zz, (void *) &ii, (void *) &m, (void *) &cnt, (void *) &seen_snapshot, (void *) &seen};
         const size_t dyn = ((size_t) (6 + 4 * cnt) * 64 + 25 * cnt) * sizeof(double);   // LargePre
-        cudaError_t ce = cudaLaunchCooperativeKernel((const void *) k_large_updates_coop, grid, dim3(threads), args, dyn, st);
+        cudaError_t ce = cudaLaunchCooperativeKernel((const void *) k_large_updates_coop<OPT>, grid, dim3(threads), args, dyn, st);
         if (ce != cudaSuccess) return ce;
         if (cnt & 1)
         {
@@ -1109,15 +1364,27 @@ inline cudaError_t launch_large_updates(LargeParams & p, const double * z, const
     for (int k = 0; k < cnt; ++k)
     {
         // slot k of the pass holds measurement i0 + k: the kernels index ids / z with (b * m + k) from the shifted base pointers
-        k_large_update<<<grid, threads, 0, st>>>(p, z + 2 * (int64_t) i0, ids + i0, m, k, p.x, p.x2, seen_snapshot, seen);
+        k_large_update<OPT><<<grid, threads, 0, st>>>(p, z + 2 * (int64_t) i0, ids + i0, m, k, p.x, p.x2, seen_snapshot, seen);
         double * tmp = p.x;
         p.x = p.x2;
         p.x2 = tmp;
     }
-    const cudaError_t re = launch_large_rank_update(p, kk, st);
+    const cudaError_t re = kJoseph ? launch_large_rank_update_sym(p, kk, st) : launch_large_rank_update(p, kk, st);
     if (re != cudaSuccess) return re;
     tail();
     return cudaGetLastError();
+}
+
+inline cudaError_t launch_large_updates(LargeParams & p, const double * z, const int32_t * ids, int m, int i0, int cnt,
+                                        const int32_t * seen_snapshot, int32_t * seen, cudaStream_t st, const LargeAssoc * assoc = nullptr)
+{
+    switch (p.options & kLargePassOpts)
+    {
+    case 0u: return launch_large_updates_t<0u>(p, z, ids, m, i0, cnt, seen_snapshot, seen, st, assoc);
+    case kOptWrapInnovation: return launch_large_updates_t<kOptWrapInnovation>(p, z, ids, m, i0, cnt, seen_snapshot, seen, st, assoc);
+    case kOptJoseph: return launch_large_updates_t<kOptJoseph>(p, z, ids, m, i0, cnt, seen_snapshot, seen, st, assoc);
+    default: return launch_large_updates_t<kLargePassOpts>(p, z, ids, m, i0, cnt, seen_snapshot, seen, st, assoc);
+    }
 }
 
 }   // namespace nuslam

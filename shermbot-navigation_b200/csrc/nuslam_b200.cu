@@ -256,6 +256,8 @@ nuslam::LargeParams make_large_params(nuslam_ekf * h)
     p.P = h->lg_P;
     p.status = h->status;
     p.strict_from = h->lg_seen_snap ? h->lg_seen_snap + h->batch : nullptr;
+    p.applied = h->lg_seen_snap ? h->lg_seen_snap + 2 * h->batch : nullptr;
+    p.options = h->cfg.options;
     memcpy(p.Q, h->cfg.Q, sizeof(p.Q));
     memcpy(p.R, h->cfg.R, sizeof(p.R));
     return p;
@@ -309,8 +311,7 @@ int large_associate(nuslam_ekf * h, const double * z, int32_t * id_out)
     if (rc) return rc;
     int32_t * result = static_cast<int32_t *>(h->lg_assoc_result.p);
     CU(cudaMemsetAsync(result, 0x7f, sizeof(int32_t) * h->batch, h->stream));
-    nuslam::k_large_associate<<<dim3((unsigned) ((p.n + 127) / 128), (unsigned) p.batch), 128, 0, h->stream>>>(
-        p, z, 1, 0, 0, h->x, h->seen, result, h->cfg.assoc_min, h->cfg.assoc_max, true);
+    nuslam::launch_large_associate(p, z, 1, 0, 0, h->x, h->seen, result, h->cfg.assoc_min, h->cfg.assoc_max, true, h->stream);
     CU(cudaGetLastError());
     nuslam::k_large_assoc_finalize<<<(unsigned) ((p.batch + 63) / 64), 64, 0, h->stream>>>(p, 1, 0, 0, h->seen, result,
                                                                                           static_cast<int32_t *>(h->lg_ids_slot.p), id_out, true);
@@ -372,11 +373,6 @@ int nuslam_ekf_create(const nuslam_ekf_config * cfg, int64_t batch, int device, 
     h->strict_warps = 4;
     while (h->strict_warps > 1 && h->strict_smem * h->strict_warps > 200 * 1024) h->strict_warps /= 2;
     if (cfg->mode == NUSLAM_MODE_LARGE || h->strict_smem * h->strict_warps > (size_t) prop.sharedMemPerBlockOptin) h->large = true;
-    if (h->large && cfg->options != 0)
-    {
-        delete h;
-        return fail(NUSLAM_ERR_UNSUPPORTED, "the NUSLAM_OPT_* variants run in the oracle-order kernels only (state too long / large-map mode)");
-    }
     // the register kernel covers n_landmarks <= 12; any larger map (that still fits on chip) runs the oracle-order CUDA kernels
     // (same results to the last bit of the reference's arithmetic, lower throughput) -- a FAST request never fails for its size
     if (!h->large && cfg->mode == NUSLAM_MODE_FAST && !nuslam::fast_supported(cfg->n_landmarks)) h->cfg.mode = NUSLAM_MODE_STRICT;
@@ -416,7 +412,8 @@ int nuslam_ekf_create(const nuslam_ekf_config * cfg, int64_t batch, int device, 
         cudaError_t l2 = cudaMalloc(&h->lg_U, sizeof(double) * 2 * nuslam::kLargeMMax * l * batch);
         cudaError_t l3 = cudaMalloc(&h->lg_V, sizeof(double) * 2 * nuslam::kLargeMMax * l * batch);
         cudaError_t l4 = cudaMalloc(&h->lg_P, sizeof(double) * 2 * l * batch);
-        cudaError_t l5 = cudaMalloc(&h->lg_seen_snap, sizeof(int32_t) * 2 * batch);   // [0, B): seen snapshot of the scan, [B, 2B): strict_from of the pass
+        // [0, B): seen snapshot of the scan, [B, 2B): strict_from of the pass, [2B, 3B): `applied` of the pass (JOSEPH)
+        cudaError_t l5 = cudaMalloc(&h->lg_seen_snap, sizeof(int32_t) * 3 * batch);
         if (l1 != cudaSuccess || l2 != cudaSuccess || l3 != cudaSuccess || l4 != cudaSuccess || l5 != cudaSuccess)
         {
             nuslam_ekf_destroy(h);
