@@ -9,6 +9,7 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdlib.h>
+#include <string.h>
 #include "ekf_strict.cuh"
 
 namespace nuslam
@@ -17,22 +18,13 @@ namespace nuslam
 constexpr int kFastMMax = 16;   // measurements per step handled by the FAST kernels
 inline bool fast_supported(int n) { return n >= 1 && n <= 12; }
 
-#ifndef NUSLAM_DEFAULT_KERNEL
-#define NUSLAM_DEFAULT_KERNEL 4   // 0 static, 1 pair, 2 fast, 3 resident (ekf_res.cuh), 4 resident pair (ekf_res2.cuh)
-#endif
-// which register kernel serves known correspondence at the BASELINE map size (NUSLAM_KERNEL, read at every call; A/B timing and
-// the equality tests): "fast" (ekf_fast.cuh, which also serves everything else), "static" (this file), "pair" (ekf_pair.cuh).
-// Measured on B200 (profiles/r02_kernel_iterations.md): the fully unrolled static schedules outgrow the instruction cache
-// (92 KB / 60 KB of code against 32 KB) and lose more to instruction fetch than they save in address arithmetic.
-inline int known_ids_kernel()
+// Known correspondence at the BASELINE map size is served by the resident pair kernel (ekf_res2.cuh). NUSLAM_KERNEL=fast hands it to
+// the register-fragment kernel (ekf_fast.cuh, which serves everything else) for A/B timing and the agreement test; unset or any other
+// value: the resident pair kernel. Read at every call, so that a process can switch between the two.
+inline bool force_fast_kernel()
 {
     const char * e = getenv("NUSLAM_KERNEL");
-    if (e && e[0] == 'p') return 1;
-    if (e && e[0] == 's') return 0;
-    if (e && e[0] == 'f') return 2;
-    // "res": ekf_res.cuh, "res2": ekf_res2.cuh, "res2a": ekf_res2.cuh + the resident pair kernel with on-device association (ekf_res2a.cuh)
-    if (e && e[0] == 'r') return (e[1] && e[2] && e[3] == '2') ? (e[4] == 'a' ? 5 : 4) : 3;
-    return NUSLAM_DEFAULT_KERNEL;
+    return e && strcmp(e, "fast") == 0;
 }
 
 struct FastLaunch

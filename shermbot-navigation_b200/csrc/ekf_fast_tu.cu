@@ -10,11 +10,7 @@
 #include "ekf_strict.cuh"
 #include "ekf_fast_api.cuh"
 #include "ekf_fast.cuh"
-#include "ekf_pair.cuh"
-#include "ekf_static.cuh"
-#include "ekf_res.cuh"
 #include "ekf_res2.cuh"
-#include "ekf_res2a.cuh"
 
 namespace nuslam
 {
@@ -30,14 +26,9 @@ namespace
 template <int OP>
 int fast_path(const FastLaunch & fl, const EkfParams & p_in, bool do_predict, cudaError_t * err, const char ** where)
 {
-    // known correspondence at the BASELINE map size: the resident pair kernel (ekf_res2.cuh; NUSLAM_KERNEL = fast / pair / static / res
-    // select the earlier kernels for A/B timing); everything else: ekf_fast.cuh
-    const int which = known_ids_kernel();
-    const bool special = which != 2 && pair_supported(fl.n_landmarks, p_in);
-    // unknown correspondence at the BASELINE map size: ekf_fast.cuh's association instantiation; NUSLAM_KERNEL=res2a selects the resident
-    // pair kernel with on-device association (ekf_res2a.cuh: same results, measured no faster -- 12 warps x 2 filters x 266 instructions
-    // per filter-measurement against 16 warps x 357: profiles/r02_kernel_iterations.md)
-    const bool assoc_pair = which == 5 && res2a_supported(fl.n_landmarks, p_in, do_predict);
+    // known correspondence at the BASELINE map size: the resident pair kernel (ekf_res2.cuh; NUSLAM_KERNEL=fast selects ekf_fast.cuh for
+    // A/B timing); everything else: ekf_fast.cuh
+    const bool res2 = !force_fast_kernel() && res2_supported(fl.n_landmarks, p_in);
     const int warps = fl.strict_warps;
     const size_t smem = fl.strict_smem * warps;
     static size_t configured_dev[kMaxDevices][8] = {{0}};
@@ -57,7 +48,7 @@ int fast_path(const FastLaunch & fl, const EkfParams & p_in, bool do_predict, cu
     if (blocks > resident) blocks = resident;
     // the resident pair kernel and the register-fragment kernel launch the list kernel themselves, behind their own grid and only when a
     // filter was handed over (ekf_strict.cuh strict_tail): a step of a built map is one launch
-    const bool tail = tail_launch_active() && !assoc_pair && (!special || which >= 4) && smem <= 48 * 1024;
+    const bool tail = tail_launch_active() && smem <= 48 * 1024;
     EkfParams p = p_in;
     if (tail)
     {
@@ -65,12 +56,8 @@ int fast_path(const FastLaunch & fl, const EkfParams & p_in, bool do_predict, cu
         p.tail_threads = warps * 32;
         p.tail_smem = (int) smem;
     }
-    const int rc = assoc_pair    ? launch_res2a_n<12>(p, do_predict, fl.sm_count, fl.worklist, fl.wl_count, fl.stream)
-                   : !special    ? launch_fast(fl.n_landmarks, p, do_predict, fl.sm_count, fl.worklist, fl.wl_count, fl.stream)
-                   : which >= 4 ? launch_res2_n<12>(p, do_predict, fl.sm_count, fl.worklist, fl.wl_count, fl.stream)
-                   : which == 3 ? launch_res_n<12>(p, do_predict, fl.sm_count, fl.worklist, fl.wl_count, fl.stream)
-                   : which == 1 ? launch_pair_n<12>(p, do_predict, fl.sm_count, fl.worklist, fl.wl_count, fl.stream)
-                                : launch_static_n<12>(p, do_predict, fl.sm_count, fl.worklist, fl.wl_count, fl.stream);
+    const int rc = res2 ? launch_res2_n<12>(p, do_predict, fl.sm_count, fl.worklist, fl.wl_count, fl.stream)
+                        : launch_fast(fl.n_landmarks, p, do_predict, fl.sm_count, fl.worklist, fl.wl_count, fl.stream);
     // not covered by the FAST kernels (more than 16 measurements per step, ragged counts with known ids, a state pointer that is not
     // 8-byte aligned): the caller runs the oracle-order kernel over the whole batch
     if (rc == -1) return -1;

@@ -1,27 +1,28 @@
 // ekf_res2.cuh -- FAST arithmetic, TWO filters per warp, both Sigma images RESIDENT IN SHARED MEMORY: fused predict + m sequential
 // updates with known correspondence (the headline kernel of BASELINE.json configs[1]).
 //
-// What the round-2 what-if builds of the one-filter resident kernel (ekf_res.cuh, profiles/r02_kernel_iterations.md) showed: the step is
-// bound by the DISPATCH port of the four warp schedulers -- an fp64 instruction occupies it for two cycles (the pipe is 16 lanes wide),
-// everything else for one: 116 fp64 + 195 other warp-instructions per update = 107 of the 150 cycles an update costs an SM, whatever the
-// occupancy (12 ... 24 warps: 400 - 415 us) and whatever the shared-memory load (80 % or 66 % of the data pipe). HBM traffic is fully
-// hidden (no traffic at all: 389 us). Half of those fp64 instructions are the per-filter scalar chain of an update (M, M^-1, sqrt d,
-// atan2, innovation, pose), which every lane of the warp evaluates redundantly. So this kernel
+// Why two filters per warp (profiles/r02_kernel_iterations.md: what-if builds of the one-filter-per-warp predecessor of this kernel,
+// measured on B200): the step is bound by the DISPATCH port of the four warp schedulers -- an fp64 instruction occupies it for two cycles
+// (the pipe is 16 lanes wide), everything else for one: 116 fp64 + 195 other warp-instructions per update = 107 of the 150 cycles an update
+// costs an SM, whatever the occupancy (12 ... 24 warps: 400 - 415 us) and whatever the shared-memory load (80 % or 66 % of the data pipe).
+// HBM traffic is fully hidden (no traffic at all: 389 us). Half of those fp64 instructions are the per-filter scalar chain of an update
+// (M, M^-1, sqrt d, atan2, innovation, pose), which every lane of the warp evaluates redundantly. So this kernel
 //   * carries filters (2 pr, 2 pr + 1) in one warp: lane (h = lane / 16, q = lane % 16) serves filter h and owns state indices q and
 //     16 + q (two vector slots). A scalar statement and every broadcast read is issued ONCE for both filters, each half-warp evaluating
-//     its own filter's chain in the same instruction; a vector statement is issued once per slot, i.e. as often per filter as before;
-//   * keeps both Sigma images in shared memory (one bulk async copy of the 16-byte aligned 2 x 5 832 B pair in, one out, in place), reads
-//     an update's landmark rows / columns straight from the image, delays the updates in chunks of CH and applies a chunk to the landmark
-//     block in place on the fp64 tensor pipe (rank-2CH DMMA pass per filter) -- the exchange of ekf_res.cuh, so no Sigma-sized state is
-//     in registers and the pair does not cost the 168 registers of the fragment pair kernel (ekf_pair.cuh);
+//     its own filter's chain in the same instruction; a vector statement is issued once per slot, i.e. as often per filter as with one
+//     filter per warp;
+//   * keeps both Sigma images RESIDENT in shared memory (one bulk async copy of the 16-byte aligned 2 x 5 832 B pair in, one out, in
+//     place), reads an update's landmark rows / columns straight from the image, delays the updates in chunks of CH and applies a chunk to
+//     the landmark block in place on the fp64 tensor pipe (rank-2CH DMMA pass per filter). So no Sigma-sized state is in registers, and
+//     two filters per warp do not cost 168 registers as they do when Sigma is held in register fragments (437 - 454 us, latency-starved);
 //   * a 64-bit shared-memory access is processed per half-warp, i.e. per filter: both halves see the conflict-free patterns of the
 //     one-filter kernel whatever their landmarks are.
 // Per filter and update: ~67 fp64 + ~70 other warp-instructions instead of 116 + 195.
-// The arithmetic of a filter is ekf_fast.cuh's statement for statement; a filter-step with a first touch / initializeLandmark, a dead
-// filter or the missing twin of an odd batch is skipped here (work list / untouched image) exactly as in ekf_pair.cuh.
+// The arithmetic of a filter is ekf_fast.cuh's statement for statement; a filter-step with a first touch / initializeLandmark is handed to
+// the strict kernel (work list), and a dead filter or the missing twin of an odd batch keeps its image untouched.
 // Reference: nuslam/src/slam_library.cpp:65-108 (predict), :263-282 (update), nuslam/src/slam.cpp:262-319 (caller protocol).
 #pragma once
-#include "ekf_res.cuh"
+#include "ekf_fast.cuh"
 
 namespace nuslam
 {
@@ -32,23 +33,10 @@ namespace nuslam
 #ifndef NUSLAM_RES2_CTAS
 #define NUSLAM_RES2_CTAS (NUSLAM_RES2_CH == 2 ? 12 : NUSLAM_RES2_CH == 3 ? 12 : 11)
 #endif
-#ifndef NUSLAM_RES2_L2PREFETCH
-#define NUSLAM_RES2_L2PREFETCH 0   // 1: pull the pair after next towards L2 (measured: no faster, 1.5 x the DRAM reads)
-#endif
-#ifndef NUSLAM_RES2_BRANCHY
-#define NUSLAM_RES2_BRANCHY 0
-#endif
-#ifndef NUSLAM_RES2_PIPE
-#define NUSLAM_RES2_PIPE 0      // 1: the state-only chain (sqrt d, atan2, innovation) of a chunk's FIRST update is issued before the in-place pass
-#endif                          //    of the previous chunk (before predict's covariance part for the first chunk): independent work for the pass
 #ifndef NUSLAM_RES2_EXP
 #define NUSLAM_RES2_EXP 0       // timing what-ifs (WRONG results): 1 no in-place pass, 2 no atan2, 3 no pending corrections, 5 no updates at all,
 #endif                          // 8 in-place pass without its DMMAs
-#ifndef NUSLAM_RES2_WARPS
-#define NUSLAM_RES2_WARPS 1     // warps (= pairs in flight) per CTA; the warps of a CTA share nothing, a CTA of W warps only saves the
-#endif                          // 1 KB of shared memory the hardware reserves per CTA (W = 13, one CTA per SM: 13 pairs per SM instead of 12)
-constexpr int kRes2CtasPerSm = NUSLAM_RES2_CTAS;
-constexpr int kRes2Warps = NUSLAM_RES2_WARPS;
+constexpr int kRes2CtasPerSm = NUSLAM_RES2_CTAS;   // one warp (= one pair in flight) per CTA
 
 template <int CH>
 struct __align__(16) Res2Smem
@@ -62,11 +50,7 @@ struct __align__(16) Res2Smem
 };
 
 template <int N, int CH>
-#ifdef NUSLAM_RES2_MAXREG
-__global__ void __maxnreg__(NUSLAM_RES2_MAXREG)
-#else
-__global__ void __launch_bounds__(32 * kRes2Warps, kRes2CtasPerSm)
-#endif
+__global__ void __launch_bounds__(32, kRes2CtasPerSm)
 k_ekf_res2_step(const EkfParams p, const int do_predict, int32_t * __restrict__ worklist, int32_t * __restrict__ wl_count)
 {
     using G = FastGeom<N>;
@@ -77,15 +61,14 @@ k_ekf_res2_step(const EkfParams p, const int do_predict, int32_t * __restrict__ 
     static_assert(NB == 3, "row permutation written for three row blocks");
     constexpr unsigned kFull = 0xffffffffu;
     constexpr int kImg = SIG * 8, kPairBytes = 2 * kImg;   // a pair is 16-byte aligned in HBM whenever the array is
-    // per warp: [the pair's two images][exchange area][mbarrier]
+    // one warp per CTA: [the pair's two images][exchange area][mbarrier]
     extern __shared__ __align__(128) unsigned char res2_dyn[];
-    constexpr int kWarpBytes = kPairBytes + (int) sizeof(Res2Smem<CH>) + 16;
     static_assert(kPairBytes % 16 == 0 && sizeof(Res2Smem<CH>) % 16 == 0, "16-byte aligned pieces");
-    unsigned char * const stage = res2_dyn + (threadIdx.x >> 5) * kWarpBytes;
+    unsigned char * const stage = res2_dyn;
     Res2Smem<CH> & f = *reinterpret_cast<Res2Smem<CH> *>(stage + kPairBytes);
     uint64_t & full_bar = *reinterpret_cast<uint64_t *>(stage + kPairBytes + sizeof(Res2Smem<CH>));
     const int lane = threadIdx.x & 31;
-    const int64_t gw0 = (int64_t) blockIdx.x * kRes2Warps + (threadIdx.x >> 5), gwn = (int64_t) gridDim.x * kRes2Warps;   // this warp, all warps
+    const int64_t gw0 = blockIdx.x, gwn = gridDim.x;   // this warp, all warps
     const int h = lane >> 4, q = lane & 15;   // vector / scalar domain: filter of this lane, index inside the half
     const int hb = 16 * h;                    // first lane of this half
     const int g = lane >> 2, t = lane & 3;    // tile domain of the in-place pass
@@ -140,11 +123,6 @@ k_ekf_res2_step(const EkfParams p, const int do_predict, int32_t * __restrict__ 
         const int64_t bf = 2 * pr + h;
         const bool has = bf < p.batch;
         const bool next = pr + gwn < npairs;
-        if (NUSLAM_RES2_L2PREFETCH && lane == 0 && pr + 2 * gwn < npairs)   // the pair after next: towards L2 while this one is computed
-        {
-            const int64_t pn = pr + 2 * gwn;
-            prefetch_l2_bulk(p.sigma + 2 * pn * SIG, (2 * pn + 1 < p.batch) ? (uint32_t) kPairBytes : (uint32_t) (kImg & ~15));
-        }
         // ---- small inputs: loaded one pair ahead (the loads of the next pair are in flight while this one is computed) ----
         double x[2] = {nx0, nx1};
         const int st0 = nst, seen0 = nseen, my_id = nid;
@@ -261,13 +239,8 @@ k_ekf_res2_step(const EkfParams p, const int do_predict, int32_t * __restrict__ 
 #else
             double zb = atan2_unit(o.dy, o.dx, rs) - th;
 #endif
-#if NUSLAM_RES2_BRANCHY
-            if (__any_sync(kFull, abs_ge_hi(zb, kHiPi)))   // the wrap is the identity inside [-pi, pi]
-                if (abs_ge_hi(zb, kHiPi)) zb = wrap_angle(zb);
-#else
             zb = wrap_angle(zb);   // the identity inside [-pi, pi]; branch-free: the update stays ONE basic block, so that the
                                    // state-only chain (rsqrt, atan2) and the covariance chain interleave
-#endif
             o.n0 = sq * (zz.x - sq), o.n1 = o.d * (zz.y - zb);
             return o;
         };
@@ -276,12 +249,6 @@ k_ekf_res2_step(const EkfParams p, const int do_predict, int32_t * __restrict__ 
             const int cv = __shfl_sync(kFull, cval, hb + (slot & 15));
             return (slot < kFastMMax) ? cv : -1;
         };
-        StateChain sc_next = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
-        if (NUSLAM_RES2_PIPE)   // the first update's chain: independent work for the register loads and predict's covariance part
-        {
-            const int cn = col_of_slot(0);
-            sc_next = state_chain(cn >= 0 ? cn : 3, 0);
-        }
         // ---- robot rows / columns: image -> registers (vector layout, two slots) ----
         double Ct[2], Cx[2], Cy[2], Rt[2], Rx[2], Ry[2];
         Ct[0] = img[q], Cx[0] = img[LEN + q], Cy[0] = img[2 * LEN + q];
@@ -372,7 +339,7 @@ k_ekf_res2_step(const EkfParams p, const int do_predict, int32_t * __restrict__ 
                 {
                     const int c = live ? cc[s] : 3;   // a half without a measurement in this slot computes on a safe index and drops the result
                     // ---- state-only part: sqrt d, bearing, innovation (:150-160, :272 no wrap) ----
-                    const StateChain sc = (NUSLAM_RES2_PIPE && s == 0) ? sc_next : state_chain(c, i0 + s);
+                    const StateChain sc = state_chain(c, i0 + s);
                     const double dx = sc.dx, dy = sc.dy, d = sc.d, dsq = sc.dsq;
                     double n0 = sc.n0, n1 = sc.n1;
                     // ---- landmark rows c, c+1 (lane = column) and columns c, c+1 (lane = row) as of the chunk's start, from the image;
@@ -458,12 +425,7 @@ k_ekf_res2_step(const EkfParams p, const int do_predict, int32_t * __restrict__ 
                     th = fma(-k0.x, n0, fma(-k0.y, n1, th));
                     px = fma(-k1.x, n0, fma(-k1.y, n1, px));
                     py = fma(-k2.x, n0, fma(-k2.y, n1, py));
-#if NUSLAM_RES2_BRANCHY
-                    if (__any_sync(kFull, abs_ge_hi(th, kHiPi)))   // slam_library.cpp:275-276 (the identity inside [-pi, pi])
-                        if (abs_ge_hi(th, kHiPi)) th = wrap_angle(th);
-#else
                     th = wrap_angle(th);   // slam_library.cpp:275-276 (the identity inside [-pi, pi])
-#endif
                     if (q == 0) x[0] = th;
 #pragma unroll
                     for (int sl = 0; sl < 2; ++sl)
@@ -494,11 +456,6 @@ k_ekf_res2_step(const EkfParams p, const int do_predict, int32_t * __restrict__ 
                     }
                     __syncwarp();   // later slots read this slot's Kt / Wt at their landmark's indices
                 }
-            }
-            if (NUSLAM_RES2_PIPE && i0 + CH < m)   // the next chunk's first state-only chain: independent of the pass below
-            {
-                const int cn = col_of_slot(i0 + CH);
-                sc_next = state_chain(cn >= 0 ? cn : 3, i0 + CH);
             }
             // (D) one pass per filter applies the chunk to the landmark block of its image in place: tile += (-Kt) Wt
             __syncwarp();
@@ -600,10 +557,9 @@ k_ekf_res2_step(const EkfParams p, const int do_predict, int32_t * __restrict__ 
 template <int N>
 int launch_res2_n(const EkfParams & p, bool do_predict, int sm_count, int32_t * worklist, int32_t * wl_count, cudaStream_t stream)
 {
-    const int64_t npairs = (p.batch + 1) / 2;
-    int64_t blocks = (npairs + kRes2Warps - 1) / kRes2Warps;
+    int64_t blocks = (p.batch + 1) / 2;   // one pair per warp
     if (blocks > kRes2CtasPerSm * (int64_t) sm_count) blocks = kRes2CtasPerSm * (int64_t) sm_count;
-    constexpr int kSmem = kRes2Warps * (2 * FastGeom<N>::SIG * 8 + (int) sizeof(Res2Smem<NUSLAM_RES2_CH>) + 16);
+    constexpr int kSmem = 2 * FastGeom<N>::SIG * 8 + (int) sizeof(Res2Smem<NUSLAM_RES2_CH>) + 16;
     static bool configured_dev[kMaxDevices] = {false};
     bool & configured = configured_dev[device_slot()];
     if (!configured)
@@ -613,8 +569,15 @@ int launch_res2_n(const EkfParams & p, bool do_predict, int sm_count, int32_t * 
         if (e != cudaSuccess) return (int) e;
         configured = true;
     }
-    k_ekf_res2_step<N, NUSLAM_RES2_CH><<<(unsigned) blocks, 32 * kRes2Warps, kSmem, stream>>>(p, do_predict ? 1 : 0, worklist, wl_count);
+    k_ekf_res2_step<N, NUSLAM_RES2_CH><<<(unsigned) blocks, 32, kSmem, stream>>>(p, do_predict ? 1 : 0, worklist, wl_count);
     return (int) cudaGetLastError();
+}
+
+// known correspondence, 16-byte aligned Sigma array, the BASELINE map size; everything else stays with ekf_fast.cuh
+inline bool res2_supported(int n, const EkfParams & p)
+{
+    return n == 12 && p.ids != nullptr && p.m_valid == nullptr && p.m >= 0 && p.m <= kFastMMax && p.batch >= 1 &&
+           (reinterpret_cast<uintptr_t>(p.sigma) & 15) == 0 && (reinterpret_cast<uintptr_t>(p.x) & 7) == 0;
 }
 
 }   // namespace nuslam

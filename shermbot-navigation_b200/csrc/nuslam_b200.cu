@@ -191,13 +191,13 @@ int launch_strict(nuslam_ekf * h, const nuslam::EkfParams & p)
 
 // FAST mode: the register / resident kernel, then the strict kernel over the filters it handed over (usually none).
 // Known correspondence: ekf_fast_tu.cu -- the kernel launches the list kernel itself, one launch per step of a built map.
-// On-device association: this unit's whole-program build of ekf_fast.cuh + a host launch of the list kernel (the relocatable build costs
-// the association kernel 1.5 %, and with unknown correspondence hand-overs -- new landmarks -- are frequent: closed loop 0.62 against
-// 0.56 ms per step, measured).
+// On-device association (ids == NULL): this unit's whole-program build of ekf_fast.cuh + a host launch of the list kernel (the
+// relocatable build costs the association kernel 1.5 %, and with unknown correspondence hand-overs -- new landmarks -- are frequent:
+// closed loop 0.62 against 0.56 ms per step, measured).
 template <int OP>
 int launch_fast_then_strict(nuslam_ekf * h, const nuslam::EkfParams & p, bool do_predict)
 {
-    if (p.ids == nullptr && nuslam::known_ids_kernel() != 5)
+    if (p.ids == nullptr)
     {
         const int rc = nuslam::launch_fast(h->cfg.n_landmarks, p, do_predict, h->sm_count, h->worklist, h->wl_count, h->stream);
         if (rc == -1) return launch_strict<OP>(h, p);

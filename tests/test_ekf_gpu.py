@@ -440,12 +440,12 @@ def test_fast_step_shapes(cuda_lib, orc, B, n, m, dropout):
 
 @pytest.mark.parametrize("B,m,dropout", [(64, 12, 0.0), (33, 12, 0.3), (7, 5, 0.0), (1, 12, 0.0), (6, 16, 0.1), (5, 16, 0.5)])
 def test_known_ids_kernels_agree(cuda_lib, orc, B, m, dropout, monkeypatch):
-    """The three register kernels that serve known correspondence at 12 landmarks -- the static-schedule kernel (ekf_static.cuh, the
-    default: slot-space permutation, unrolled updates), the two-filters-per-warp kernel (ekf_pair.cuh) and the dynamic one
-    (ekf_fast.cuh) -- evaluate the same arithmetic in different layouts and slot orders: the same scenario through all three
-    (NUSLAM_KERNEL, read at every call) must agree to rounding -- odd batches, dropped measurements (id 0), fewer measurements than
-    landmarks and m > n (repeated landmarks, or measurements in slots beyond the map: the oracle-order kernel takes those steps)
-    included -- and every one sits within 1e-9 of the oracle."""
+    """The two kernels that serve known correspondence at 12 landmarks -- the resident pair kernel (ekf_res2.cuh, the default: two
+    filters per warp, Sigma images in shared memory, delayed chunks applied in place) and the register-fragment kernel (ekf_fast.cuh,
+    NUSLAM_KERNEL=fast, read at every call) -- evaluate the same arithmetic in different layouts and update orders: the same scenario
+    through both must agree to rounding -- odd batches, dropped measurements (id 0), fewer measurements than landmarks and m > n
+    (repeated landmarks, or measurements in slots beyond the map: the oracle-order kernel takes those steps) included -- and each sits
+    within 1e-9 of the oracle."""
     n, T = 12, 10
     sc = synth.ekf_scenario(B, T, n=n, seed=300 + B + m)
     rng = np.random.default_rng(B * 17 + m)
@@ -468,7 +468,7 @@ def test_known_ids_kernels_agree(cuda_lib, orc, B, m, dropout, monkeypatch):
     first = orc.ekf_run(n, sc["robot0"], sc["map0"], sc["Q"], sc["R"], sc["twists"][:1], sc["z"][:1], sc["ids"][:1])
     want = orc.ekf_run(n, sc["robot0"], sc["map0"], sc["Q"], sc["R"], sc["twists"][1:], z[1:], ids[1:], init=(first["x"], first["sigma"], first["seen"]))
     out = {}
-    for kern in ("static", "pair", "res", "res2", "fast"):
+    for kern in ("res2", "fast"):
         monkeypatch.setenv("NUSLAM_KERNEL", kern)
         eng = cuda_lib.BatchedExtendedKalman(sc["robot0"], sc["map0"], sc["Q"], sc["R"], mode="fast")
         eng.set_state(first["x"], first["sigma"], first["seen"])
@@ -479,14 +479,13 @@ def test_known_ids_kernels_agree(cuda_lib, orc, B, m, dropout, monkeypatch):
         assert not status.any() and np.array_equal(seen, want["seen"])
         assert rel_max(x, want["x"]) < TOL and max(rel_max(s[b], want["sigma"][b]) for b in range(B)) < TOL, kern
     x0, s0, _, _ = out["fast"]
-    for kern in ("static", "pair", "res", "res2"):
-        x1, s1, _, _ = out[kern]
-        ex, es = rel_max(x1, x0), max(rel_max(s1[b], s0[b]) for b in range(B))
-        print(f"[{kern} vs fast, B={B} m={m} dropout={dropout}] x rel {ex:.2e}, Sigma rel {es:.2e}")
-        # the kernels round a few terms of the 2 x 2 part differently (~1e-13 after 9 steps); steps that go to the oracle-order kernel in
-        # one of them (m > n) differ by its arithmetic
-        tol = 1e-11 if m <= n else 1e-10
-        assert ex < tol and es < tol
+    x1, s1, _, _ = out["res2"]
+    ex, es = rel_max(x1, x0), max(rel_max(s1[b], s0[b]) for b in range(B))
+    print(f"[res2 vs fast, B={B} m={m} dropout={dropout}] x rel {ex:.2e}, Sigma rel {es:.2e}")
+    # the kernels round a few terms of the 2 x 2 part differently (~1e-13 after 9 steps); steps that go to the oracle-order kernel in
+    # one of them (m > n) differ by its arithmetic
+    tol = 1e-11 if m <= n else 1e-10
+    assert ex < tol and es < tol
 
 
 @pytest.mark.parametrize("B,n", [(64, 12), (16, 6), (12, 8), (10, 3), (9, 10)])

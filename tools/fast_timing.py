@@ -1,6 +1,7 @@
 #!/usr/bin/env python
-"""Per-phase clock64 breakdown of the FAST kernel (block 0, warp 0). Needs a -DNUSLAM_TIMING build:
-   NUSLAM_B200_LIB=build/variants/lib_timing.so python tools/fast_timing.py"""
+"""Per-phase clock64 breakdown of the FAST kernel (ekf_fast.cuh, block 0, warp 0). Needs a -DNUSLAM_TIMING build, and NUSLAM_KERNEL=fast:
+   at 12 landmarks the default is the resident pair kernel (ekf_res2.cuh), which has no timing hooks.
+   NUSLAM_KERNEL=fast NUSLAM_B200_LIB=build/variants/lib_timing.so python tools/fast_timing.py"""
 import ctypes as C
 import os, sys
 from pathlib import Path
@@ -31,11 +32,8 @@ eng.synchronize()
 lib.nuslam_debug_fast_timing(out, 0)
 v = np.array(list(out), dtype=np.float64)
 nblk = 148 * int(os.environ.get("NUSLAM_FAST_CTAS_PER_SM", "16"))
-per_warp = int(os.environ.get("NUSLAM_FILTERS_PER_WARP", "1"))   # 2: the pair kernel
-filters = K * per_warp * ((B // per_warp + nblk - 1) // nblk)   # filters processed by block 0 / warp 0
+filters = K * ((B + nblk - 1) // nblk)   # filters processed by block 0 / warp 0
 names = ["load", "predict", "publish", "pre (Pt,Wt)", "2x2 part + Kt", "post (x, robot)", "dmma", "store"]
-if per_warp == 2:
-    names = ["inputs + perm + wait", "load regs + predict", "publish", "V1 (Pt,Wt)", "2x2 part + Kt + cols", "pose + rows", "dmma", "store"]
 tot = v[:8].sum()
 print(f"block 0 / warp 0: {filters} filter-steps, {tot / filters:.0f} cycles per filter-step ({tot / filters / 12:.0f} per update)")
 for k, nm in enumerate(names):
