@@ -425,7 +425,10 @@ k_ekf_res2_step(const EkfParams p, const int do_predict, int32_t * __restrict__ 
                     th = fma(-k0.x, n0, fma(-k0.y, n1, th));
                     px = fma(-k1.x, n0, fma(-k1.y, n1, px));
                     py = fma(-k2.x, n0, fma(-k2.y, n1, py));
-                    th = wrap_angle(th);   // slam_library.cpp:275-276 (the identity inside [-pi, pi])
+                    // slam_library.cpp:275-276 (the identity inside [-pi, pi]), only where this filter had the update: a half with no
+                    // measurement in this slot (its partner has one) keeps a heading that predict carried outside [-pi, pi], as the
+                    // reference does; wrapping it anyway made the state depend on the partner filter
+                    if (ok) th = wrap_angle(th);
                     if (q == 0) x[0] = th;
 #pragma unroll
                     for (int sl = 0; sl < 2; ++sl)

@@ -41,7 +41,7 @@ __device__ __forceinline__ double div_fast(double a, double b)
     return fma(fma(-b, q, a), y, q);
 }
 
-// 1/sqrt(x): MUFU.RSQ64H seed + 2 Newton steps
+// 1/sqrt(x): MUFU.RSQ64H seed + 2 Newton steps -> <= 1 ulp for normal x
 __device__ __forceinline__ double rsqrt_fast(double x)
 {
     double y;
@@ -53,8 +53,8 @@ __device__ __forceinline__ double rsqrt_fast(double x)
     return y;
 }
 
-// 1/sqrt(x) with ONE Newton step (relative error ~1e-12): enough where a consumer squares the error away -- sqrt(x) = x rs refined once
-// is exact to an ulp -- or tolerates it (the unit vector of atan2_unit: <= 1e-14 rad)
+// 1/sqrt(x) with ONE Newton step (relative error <= 1.3e-12, worst measured 1.23e-12): enough where a consumer squares the error
+// away -- sqrt(x) = x rs refined once is exact to an ulp -- or tolerates it (the unit vector of atan2_unit: <= 1e-14 rad)
 __device__ __forceinline__ double rsqrt_1(double x)
 {
     double y;
@@ -68,6 +68,11 @@ __device__ __forceinline__ double rsqrt_1(double x)
 //   atan(mn / mx) = atan(t_k) + atan(r),   r = (mn - t_k mx) / (mx + t_k mn),   |r| <= ~1 / 100,
 // so a degree-7 odd polynomial (error r^9 / 9 < 1e-19) finishes it; atan(t_k) comes from a 65-entry (hi, lo) table and the
 // octant (|y| > |x|, x < 0, y < 0) from an 8-entry table: atan2 = A + S (atan(t_k) + atan(r)) with A = k pi/4 (hi + lo).
+// Domain: max(|x|, |y|) in [2^-100, 2^100] (its callers pass metres: the bearing of the large-map model, the circle fit's inscribed
+// angles); there the error is <= 2 ulp (worst measured 1.36 ulp). Outside it the fp32 estimate of mn / mx breaks down ((float) mx
+// overflows or is denormal, __fdividef returns 0 for a divisor above 2^126), k is wrong, |r| is no longer small and the result is a
+// number far from atan2 (NaN for a denormal mx, which rcp_fast flushes to zero); nothing traps. The signs are tested with x < 0 and
+// y < 0, so a zero argument counts as +0: atan2_fast(-0, x < 0) = +pi (libm: -pi), atan2_fast(y, -0) = atan2(y, +0).
 struct AtanOctant
 {
     double hi, lo, s, pad;
@@ -279,8 +284,10 @@ __device__ __forceinline__ double atan2_unit(double y, double x, double rs)
 
 // sin and cos without a slow path (no call into the device library: under -rdc such a call is an ABI call that costs the FAST kernels
 // registers). Cody-Waite reduction by pi/2 in three 33-bit pieces (exact products for |a| < ~1e6; beyond that the error grows with |a|,
-// a heading is normalised to [-pi, pi] after every update), then the fdlibm kernels on [-pi/4, pi/4] (|error| < 2^-58): <= 1 ulp of
-// the library's results on the headings an EKF sees, far inside FAST mode's 1e-9.
+// a heading is normalised to [-pi, pi] after every update), then the fdlibm kernels on [-pi/4, pi/4] (|error| < 2^-58). Against the
+// correctly rounded sin / cos: <= 1.7 ulp for |a| <= 1e3 (worst measured 1.63 ulp), <= 2 ulp at |a| ~ 1e6 (measured 1.94): the reduced
+// argument is rounded once before the ~0.5 ulp kernels, so this is ~1 ulp of the library's results, not of the true values; far inside
+// FAST mode's 1e-9. Pure fma arithmetic: the host computes the device's bits (tests/test_fastmath_tables.py checks it there).
 __host__ __device__ __forceinline__ void sincos_fast(double a, double * sn, double * cs)
 {
     const double k = rint(a * 6.36619772367581382433e-01);
@@ -302,7 +309,7 @@ __host__ __device__ __forceinline__ void sincos_fast(double a, double * sn, doub
 }
 
 // sin and cos of a SMALL angle (|a| <= 0.25: a wheel-odometry step) straight from the Taylor series, no argument reduction; the
-// truncation error is below 3e-18. Larger arguments take the library path.
+// truncation error is below 3e-18 and the result within 1 ulp of the correctly rounded value. Larger arguments take sincos_fast.
 static __constant__ double kSinK[6] = {-1.0 / 6.0, 1.0 / 120.0, -1.0 / 5040.0, 1.0 / 362880.0, -1.0 / 39916800.0, 1.0 / 6227020800.0};
 static __constant__ double kCosK[7] = {-0.5, 1.0 / 24.0, -1.0 / 720.0, 1.0 / 40320.0, -1.0 / 3628800.0, 1.0 / 479001600.0, -1.0 / 87178291200.0};
 __device__ __forceinline__ void sincos_small(double a, double * sn, double * cs)
