@@ -45,20 +45,11 @@ namespace nuslam
 {
 
 constexpr int kFastThreads = 32;                   // one warp = one filter in flight per CTA: no cross-warp state at all
-#ifndef NUSLAM_FAST_CTAS
-#define NUSLAM_FAST_CTAS 16
-#endif
-#ifndef NUSLAM_EXP
-#define NUSLAM_EXP 0   // timing experiments only (wrong results): 1 no atan2, 2 no publish stores, 3 no DMMA, 4 no robot-vector updates, 5 no predict
-#endif
-#ifndef NUSLAM_ASSOC_DFMA
-#define NUSLAM_ASSOC_DFMA 0   // 1: the association instantiation applies its rank-2 update per measurement by plain FMAs instead of half-empty DMMAs
-#endif
 #ifndef NUSLAM_FAST_SINGLE_STAGE
 #define NUSLAM_FAST_SINGLE_STAGE 0   // 1: one staging buffer per CTA (input image -> exchange area -> output image): half the shared memory
 #endif
 constexpr bool kFastSingleStage = NUSLAM_FAST_SINGLE_STAGE != 0;
-constexpr int kFastCtasPerSm = NUSLAM_FAST_CTAS;   // 16 single-warp CTAs / SM at 128 registers (20 at 96 registers spill; measured slower)
+constexpr int kFastCtasPerSm = 16;   // 16 single-warp CTAs / SM at 128 registers (20 at 96 registers spill; measured slower)
 
 // N > 0: the number of landmarks is a compile-time constant (the BASELINE sizes 12 and 6: every index folds). N < 0: a GENERIC
 // instantiation for any n with ceil(2 n / 8) = -N fragment blocks per side (n read from the parameters at run time; n <= 4, 8, 12
@@ -387,7 +378,7 @@ k_ekf_fast_step(const EkfParams p, const int do_predict, int32_t * __restrict__ 
         NUSLAM_T(0)
 
         // ---- predict (slam_library.cpp:65-108), oracle operation order, vector layout only ----
-        if (do_predict && NUSLAM_EXP != 5)
+        if (do_predict)
         {
             const double dth = __shfl_sync(kFull, my_tw, 0), dxx = __shfl_sync(kFull, my_tw, 1);
             // predictEstimate :71-94, then the two Jacobian entries of getA :127-148 (theta read AFTER the motion update,
@@ -599,11 +590,7 @@ k_ekf_fast_step(const EkfParams p, const int do_predict, int32_t * __restrict__ 
             if (csel) cdst[8 * q] = make_double2(C[q][b < NB ? b : 0][0], C[q][b < NB ? b : 0][1]);                        \
         }                                                                                                                  \
     }
-#if NUSLAM_EXP == 2
-                    if (bsel == 7)
-#else
                     if (bsel == 0)
-#endif
                     {
                         NUSLAM_PUBLISH(0)
                     }
@@ -669,14 +656,6 @@ k_ekf_fast_step(const EkfParams p, const int do_predict, int32_t * __restrict__ 
                     f.wt[s][lane] = make_double2(W0, W1);
                     __syncwarp();
                     NUSLAM_T(3)
-#if NUSLAM_EXP == 6
-                    // what-if: the 2 x 2 part arrives from elsewhere (a response read back from shared memory); timing only
-                    const double2 g0 = f.wt[s][0], g1 = f.wt[s][1], g2 = f.wt[s][2];
-                    const double2 q0 = g0, q1 = g1, q2 = g2;
-                    const double m00 = 1.0 + 1e-9 * q0.x, m01 = 1e-9 * q0.y, m10 = 1e-9 * q1.x, m11 = 1.0 + 1e-9 * q1.y;
-                    const double idet = 1.0 + 1e-9 * q2.x;
-                    const double n0 = 1e-6 * (zz.x - dx), n1 = 1e-6 * (zz.y - dy) + 1e-12 * q2.y;
-#else
                     // the 2 x 2 part, evaluated by every lane: M = Wt Ht^T + D^-1 R D^-1, Minv, innovation (:150-160, :272 no wrap)
                     const double2 g0 = f.wt[s][0], g1 = f.wt[s][1], g2 = f.wt[s][2], g3 = f.wt[s][c], g4 = f.wt[s][c + 1];
                     const double e0 = g3.x - g1.x, f0 = g4.x - g2.x, e1 = g3.y - g1.y, f1 = g4.y - g2.y;
@@ -691,14 +670,9 @@ k_ekf_fast_step(const EkfParams p, const int do_predict, int32_t * __restrict__ 
                     const double idet = rcp_fast(det);
                     // the bearing chain (atan2, wrap) is independent of the Minv chain: evaluated before the branch so that the two
                     // dependency chains interleave
-#if NUSLAM_EXP == 1
-                    const double zb = zz.y - 1e-3 * dy;
-#else
                     double zb = atan2_unit(dy, dx, rs) - th;
                     if (abs_ge_hi(zb, kHiPi)) zb = wrap_angle(zb);   // the identity inside [-pi, pi]
-#endif
                     const double n0 = sq * (zz.x - sq), n1 = d * (zz.y - zb);
-#endif
                     if (!abs_ge_hi(idet, kHi1e300))   // |idet| < ~1e300: warp-uniform; false for det = 0, inf or nan, where arma::inv throws (slam_library.cpp:270)
                     {
                         done = true;
@@ -718,14 +692,12 @@ k_ekf_fast_step(const EkfParams p, const int do_predict, int32_t * __restrict__ 
                         if (lane == 0) x = th;
                         f.xs[lane + 1] = x;
                         // robot rows / columns: Sigma -= Kt Wt restricted to them
-#if NUSLAM_EXP != 4
                         Rt = fma(k0.x, W0, fma(k0.y, W1, Rt));
                         Rx = fma(k1.x, W0, fma(k1.y, W1, Rx));
                         Ry = fma(k2.x, W0, fma(k2.y, W1, Ry));
                         Ct = fma(nk0, g0.x, fma(nk1, g0.y, Ct));
                         Cx = fma(nk0, g1.x, fma(nk1, g1.y, Cx));
                         Cy = fma(nk0, g2.x, fma(nk1, g2.y, Cy));
-#endif
                         __syncwarp();
                         NUSLAM_T(5)
                     }
@@ -740,29 +712,8 @@ k_ekf_fast_step(const EkfParams p, const int do_predict, int32_t * __restrict__ 
                     __syncwarp();
                 }
             }
-            // (D) one DMMA pass applies the chunk to the fragments: C += (-Kt) Wt, k = (u0, u1, v0, v1)
-            if (ASSOC && NUSLAM_ASSOC_DFMA)
-            {
-                // one measurement per pass: half of a DMMA's k would be empty, and the fp64 pipe takes as long for an m8n8k4 DMMA as for
-                // eight DFMAs -- the rank-2 update of the 18 fragment entries by 36 plain FMAs holds it half as long as the 9 DMMAs
-                double2 ka2[NB], w0[NB], w1[NB];
-#pragma unroll
-                for (int bb = 0; bb < NB; ++bb)
-                {
-                    ka2[bb] = f.kt[0][3 + 8 * bb + g];
-                    w0[bb] = f.wt[0][3 + 8 * bb + 2 * t];
-                    w1[bb] = f.wt[0][3 + 8 * bb + 2 * t + 1];
-                }
-#pragma unroll
-                for (int br = 0; br < NB; ++br)
-#pragma unroll
-                    for (int bc = 0; bc < NB; ++bc)
-                    {
-                        C[br][bc][0] = fma(ka2[br].x, w0[bc].x, fma(ka2[br].y, w0[bc].y, C[br][bc][0]));
-                        C[br][bc][1] = fma(ka2[br].x, w1[bc].x, fma(ka2[br].y, w1[bc].y, C[br][bc][1]));
-                    }
-            }
-            else
+            // (D) one DMMA pass applies the chunk to the fragments: C += (-Kt) Wt, k = (u0, u1, v0, v1). Its operands live in a scope of
+            // their own and die with the pass (without the scope the compiler allocates the NB = 1 instantiations' registers differently)
             {
                 const double * ka = reinterpret_cast<const double *>(&f.kt[t >> 1][3 + g]) + (t & 1);
                 const double * wa = reinterpret_cast<const double *>(&f.wt[t >> 1][3 + g]) + (t & 1);
@@ -776,15 +727,7 @@ k_ekf_fast_step(const EkfParams p, const int do_predict, int32_t * __restrict__ 
 #pragma unroll
                 for (int br = 0; br < NB; ++br)
 #pragma unroll
-                    for (int bc = 0; bc < NB; ++bc)
-                    {
-#if NUSLAM_EXP == 3
-                        C[br][bc][0] += a[br];
-                        C[br][bc][1] += b[bc];
-#else
-                        dmma884(C[br][bc][0], C[br][bc][1], a[br], b[bc]);
-#endif
-                    }
+                    for (int bc = 0; bc < NB; ++bc) dmma884(C[br][bc][0], C[br][bc][1], a[br], b[bc]);
             }
             __syncwarp();
             NUSLAM_T(6)

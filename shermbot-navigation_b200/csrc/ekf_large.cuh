@@ -845,10 +845,8 @@ __device__ __forceinline__ void dmma884_large(double & c0, double & c1, double a
 // Sigma <- Sigma - K W with K = U^T (len x 2m), W = V (2m x len): CTA tile 64 x 64 (4 warps of 32 x 32), operands staged in
 // shared memory, accumulators initialised from Sigma. kk = padded 2m (multiple of 4).
 constexpr int kLargeTile = 64;
-#ifndef NUSLAM_LARGE_RANK_CTAS
-#define NUSLAM_LARGE_RANK_CTAS 4   // resident CTAs per SM the register allocation aims at (3 at 148 registers: measured slower at rank >= 24)
-#endif
-__global__ void __launch_bounds__(128, NUSLAM_LARGE_RANK_CTAS) k_large_rank_update(const LargeParams p, int kk)
+constexpr int kRankCtas = 4;   // resident CTAs per SM the register allocation aims at (3 at 148 registers: measured slower at rank >= 24)
+__global__ void __launch_bounds__(128, kRankCtas) k_large_rank_update(const LargeParams p, int kk)
 {
     __shared__ double su[2 * kLargeMMax][kLargeTile + 1];   // -K: su[k][r]
     __shared__ double sv[2 * kLargeMMax][kLargeTile + 1];   //  W: sv[k][c]
@@ -919,16 +917,7 @@ __global__ void __launch_bounds__(128, NUSLAM_LARGE_RANK_CTAS) k_large_rank_upda
 // (Two stages per CTA at three CTAs per SM -- 96 KB in flight -- were measured slower than the plain kernel: 0.28 ms at rank 4.)
 constexpr int kRankStageLd = kLargeTile + 2;   // column stride of a stage in doubles (66: 2 x 66 = 4 mod 16, the four t of a half-warp hit disjoint banks)
 constexpr int kRankStageDoubles = kLargeTile * kRankStageLd;
-#ifndef NUSLAM_LARGE_RANK_PIPE
-#define NUSLAM_LARGE_RANK_PIPE 1
-#endif
-#ifndef NUSLAM_LARGE_PIPE_SMEM_OPS
-#define NUSLAM_LARGE_PIPE_SMEM_OPS 0   // (measured slower: m = 12 scan 0.454 ms against 0.345) 1: the tile's K / W operands staged in shared memory (requested before the wait for the tile, read by LDS in the k-loop); 3 CTAs per SM
-#endif
-#ifndef NUSLAM_LARGE_PIPE_CTAS
-#define NUSLAM_LARGE_PIPE_CTAS (NUSLAM_LARGE_PIPE_SMEM_OPS ? 3 : 4)
-#endif
-constexpr int kRankPipeCtas = NUSLAM_LARGE_PIPE_CTAS;
+constexpr int kRankPipeCtas = 4;   // resident CTAs per SM (3 measured 0.7 % slower)
 __global__ void __launch_bounds__(128, kRankPipeCtas) k_large_rank_update_pipe(const LargeParams p, int kk, int tiles)
 {
     extern __shared__ __align__(16) double rank_stage[];   // [64 columns][66]
@@ -959,9 +948,8 @@ __global__ void __launch_bounds__(128, kRankPipeCtas) k_large_rank_update_pipe(c
         }
         asm volatile("cp.async.commit_group;" ::: "memory");
     };
-#ifndef NUSLAM_LARGE_PIPE_L1PF
-#define NUSLAM_LARGE_PIPE_L1PF 2   // (measured: m = 32 scan 0.788 -> 0.775 -> 0.768 ms for 0 / 1 / 2, m = 12 within 1 %) pull a tile's K / W operands (kk x 64 doubles each) towards L1 ahead of the DMMAs: 1 at the top of its own round, 2 one round ahead
-#endif
+    // pull a tile's K / W operands (kk x 64 doubles each) towards L1 one round ahead of its DMMAs (measured: m = 32 scan 0.788 ms with
+    // no prefetch, 0.775 prefetched at the top of the tile's own round, 0.768 one round ahead; m = 12 within 1 %)
     auto prefetch_ops = [&](int64_t tl) {
         const int b = (int) (tl / ((int64_t) tiles * tiles));
         const int rem = (int) (tl % ((int64_t) tiles * tiles));
@@ -981,42 +969,8 @@ __global__ void __launch_bounds__(128, kRankPipeCtas) k_large_rank_update_pipe(c
     if (tile < ntiles) issue(tile);
     for (; tile < ntiles; tile += gridDim.x)
     {
-        if (NUSLAM_LARGE_PIPE_L1PF == 1) prefetch_ops(tile);
-#if NUSLAM_LARGE_PIPE_SMEM_OPS
-        // this tile's operands: requested now (their L2 latency runs under the wait for the tile), stored to shared memory behind the barrier
-        double (*su)[kLargeTile + 1] = reinterpret_cast<double (*)[kLargeTile + 1]>(rank_stage + kRankStageDoubles);
-        double (*sv)[kLargeTile + 1] = su + 2 * kLargeMMax;
-        double ur[kLargeMMax], vr[kLargeMMax];
-        {
-            const int b = (int) (tile / ((int64_t) tiles * tiles));
-            const int rem = (int) (tile % ((int64_t) tiles * tiles));
-            const int c0 = (rem / tiles) * kLargeTile, r0 = (rem % tiles) * kLargeTile;
-            const double * U = p.U + (int64_t) b * 2 * kLargeMMax * len;
-            const double * V = p.V + (int64_t) b * 2 * kLargeMMax * len;
-            const int o = threadIdx.x & 63, kh = threadIdx.x >> 6;   // element o of rows kh, kh + 2, ...
-#pragma unroll
-            for (int i = 0; i < kLargeMMax; ++i)
-            {
-                const int k = kh + 2 * i;
-                ur[i] = (k < kk && r0 + o < len) ? -__ldg(U + (int64_t) k * len + r0 + o) : 0.0;
-                vr[i] = (k < kk && c0 + o < len) ? __ldg(V + (int64_t) k * len + c0 + o) : 0.0;
-            }
-        }
-#endif
         asm volatile("cp.async.wait_group 0;" ::: "memory");
         __syncthreads();
-#if NUSLAM_LARGE_PIPE_SMEM_OPS
-        {
-            const int o = threadIdx.x & 63, kh = threadIdx.x >> 6;
-#pragma unroll
-            for (int i = 0; i < kLargeMMax; ++i)
-                if (kh + 2 * i < kk)
-                {
-                    su[kh + 2 * i][o] = ur[i];
-                    sv[kh + 2 * i][o] = vr[i];
-                }
-        }
-#endif
         double C[4][4][2];
 #pragma unroll
         for (int br = 0; br < 4; ++br)
@@ -1028,7 +982,7 @@ __global__ void __launch_bounds__(128, kRankPipeCtas) k_large_rank_update_pipe(c
         if (tile + gridDim.x < ntiles)
         {
             issue(tile + gridDim.x);
-            if (NUSLAM_LARGE_PIPE_L1PF == 2) prefetch_ops(tile + gridDim.x);
+            prefetch_ops(tile + gridDim.x);
         }
         const int b = (int) (tile / ((int64_t) tiles * tiles));
         const int rem = (int) (tile % ((int64_t) tiles * tiles));
@@ -1036,43 +990,23 @@ __global__ void __launch_bounds__(128, kRankPipeCtas) k_large_rank_update_pipe(c
         double * S = p.sigma + (int64_t) b * len * len;
         const double * U = p.U + (int64_t) b * 2 * kLargeMMax * len;
         const double * V = p.V + (int64_t) b * 2 * kLargeMMax * len;
-        // operands in fragment layout straight from L2 / L1: a = -K(row, k0 + t), b = W(k0 + t, column); rows / columns beyond len: 0
-#ifndef NUSLAM_LARGE_PIPE_KSTEPS
-#define NUSLAM_LARGE_PIPE_KSTEPS 1   // k-steps whose operands are requested together; 2 and 3 measured slower (m = 12 scan 0.408 / 0.419 ms against 0.348)
-#endif
-        constexpr int KS = NUSLAM_LARGE_PIPE_KSTEPS;
-        for (int k0 = 0; k0 < kk; k0 += 4 * KS)
+        // operands in fragment layout straight from L2 / L1: a = -K(row, k0 + t), b = W(k0 + t, column); rows / columns beyond len: 0.
+        // One k-step's operands are requested at a time: two or three together measured slower (m = 12 scan 0.408 / 0.419 ms against 0.348)
+        for (int k0 = 0; k0 < kk; k0 += 4)
         {
-            double a[KS][4], bb[KS][4];
+            const double * Uk = U + (int64_t) (k0 + t) * len + r0 + lr + g;
+            const double * Vk = V + (int64_t) (k0 + t) * len + c0 + lc + g;
+            double a[4], bb[4];
 #pragma unroll
-            for (int ks = 0; ks < KS; ++ks)
+            for (int q = 0; q < 4; ++q)
             {
-                const bool on = k0 + 4 * ks < kk;   // kk is a multiple of 4, not of 4 KS
-                const double * Uk = U + (int64_t) (k0 + 4 * ks + t) * len + r0 + lr + g;
-                const double * Vk = V + (int64_t) (k0 + 4 * ks + t) * len + c0 + lc + g;
-#pragma unroll
-                for (int q = 0; q < 4; ++q)
-                {
-#if NUSLAM_LARGE_PIPE_SMEM_OPS
-                    (void) Uk;
-                    (void) Vk;
-                    a[ks][q] = on ? su[k0 + 4 * ks + t][lr + 8 * q + g] : 0.0;
-                    bb[ks][q] = on ? sv[k0 + 4 * ks + t][lc + 8 * q + g] : 0.0;
-#else
-                    a[ks][q] = (on && r0 + lr + 8 * q + g < len) ? -__ldg(Uk + 8 * q) : 0.0;
-                    bb[ks][q] = (on && c0 + lc + 8 * q + g < len) ? __ldg(Vk + 8 * q) : 0.0;
-#endif
-                }
+                a[q] = (r0 + lr + 8 * q + g < len) ? -__ldg(Uk + 8 * q) : 0.0;
+                bb[q] = (c0 + lc + 8 * q + g < len) ? __ldg(Vk + 8 * q) : 0.0;
             }
 #pragma unroll
-            for (int ks = 0; ks < KS; ++ks)
-                if (k0 + 4 * ks < kk)
-                {
+            for (int br = 0; br < 4; ++br)
 #pragma unroll
-                    for (int br = 0; br < 4; ++br)
-#pragma unroll
-                        for (int bc = 0; bc < 4; ++bc) dmma884_large(C[br][bc][0], C[br][bc][1], a[ks][br], bb[ks][bc]);
-                }
+                for (int bc = 0; bc < 4; ++bc) dmma884_large(C[br][bc][0], C[br][bc][1], a[br], bb[bc]);
         }
 #pragma unroll
         for (int br = 0; br < 4; ++br)
@@ -1091,20 +1025,17 @@ __global__ void __launch_bounds__(128, kRankPipeCtas) k_large_rank_update_pipe(c
 inline cudaError_t launch_large_rank_update(const LargeParams & p, int kk, cudaStream_t st)
 {
     const unsigned tiles = (p.len + kLargeTile - 1) / kLargeTile;
-#if NUSLAM_LARGE_RANK_PIPE
-    // measured at 4 096 landmarks (tools/gpu_round2_ag.sh): rank 4: plain 0.20 ms, pipelined 0.23 ms; rank 24: 0.30 / 0.27 ms; rank 32: 0.37 / 0.33 ms
-    static const int pipe_min_rank = [] {
-        const char * e = getenv("NUSLAM_LARGE_PIPE_MIN_RANK");   // A/B timing
-        return e ? atoi(e) : 16;
-    }();
-    if (kk < pipe_min_rank)
+    // the plain kernel below rank 16, the pipelined one from there up. Measured at 4 096 landmarks (tools/gpu_round2_ag.sh): rank 4: plain
+    // 0.20 ms, pipelined 0.23 ms; rank 24: 0.30 / 0.27 ms; rank 32: 0.37 / 0.33 ms
+    constexpr int kPipeMinRank = 16;
+    if (kk < kPipeMinRank)
     {
         k_large_rank_update<<<dim3(tiles, tiles, (unsigned) p.batch), 128, 0, st>>>(p, kk);
         return cudaGetLastError();
     }
     static int sms_dev[kMaxDevices] = {0};
     int & sms = sms_dev[device_slot()];
-    constexpr int kSmem = (kRankStageDoubles + (NUSLAM_LARGE_PIPE_SMEM_OPS ? 2 * 2 * kLargeMMax * (kLargeTile + 1) : 0)) * (int) sizeof(double);
+    constexpr int kSmem = kRankStageDoubles * (int) sizeof(double);
     if (sms == 0)
     {
         int dev = 0, n = 0;
@@ -1117,9 +1048,6 @@ inline cudaError_t launch_large_rank_update(const LargeParams & p, int kk, cudaS
     int64_t blocks = (int64_t) tiles * tiles * p.batch;
     if (blocks > kRankPipeCtas * (int64_t) sms) blocks = kRankPipeCtas * (int64_t) sms;
     k_large_rank_update_pipe<<<(unsigned) blocks, 128, kSmem, st>>>(p, kk, (int) tiles);
-#else
-    k_large_rank_update<<<dim3(tiles, tiles, (unsigned) p.batch), 128, 0, st>>>(p, kk);
-#endif
     return cudaGetLastError();
 }
 

@@ -465,18 +465,10 @@ struct ClusterFit
 };
 constexpr int kFitNMax = 32;        // clusters up to this many points are fitted one per THREAD (work matrix interleaved in shared memory)
 constexpr int kFitThreads = 64;
-#ifndef NUSLAM_BIGS_CTAS
-#define NUSLAM_BIGS_CTAS 5   // resident CTAs (of 4 warps) per SM of the first warp-per-cluster class (96 registers per thread; measured best of 4 / 5)
-#endif
+constexpr int kBigSmallCtas = 5;    // resident CTAs (of 4 warps) per SM of the first warp-per-cluster class (96 registers per thread; measured best of 4 / 5)
 constexpr int kFitBigSmall = 126;   // largest cluster of the first warp-per-cluster class
-#ifndef NUSLAM_FIT_SMALL
-#define NUSLAM_FIT_SMALL 12
-#endif
-#ifndef NUSLAM_FIT_CTAS
-#define NUSLAM_FIT_CTAS 8
-#endif
-constexpr int kFitCtas = NUSLAM_FIT_CTAS;     // CTAs of the first class per SM
-constexpr int kFitSmall = NUSLAM_FIT_SMALL;   // largest cluster of the first size class (work matrix kFitSmall x 4 doubles per thread)
+constexpr int kFitCtas = 8;     // CTAs of the first class per SM
+constexpr int kFitSmall = 12;   // largest cluster of the first size class (work matrix kFitSmall x 4 doubles per thread)
 constexpr int kMaxFastClusters = 32;   // scans returning more clusters than this take the one-warp-per-scan path
 
 struct ScanPipe
@@ -941,7 +933,7 @@ __device__ inline void svd_n4_warp(double * A, int m, double * prod, int lane, d
 // Two capacities: up to kFitBigSmall points (7 KB of shared memory per warp: four times the resident warps, which is what hides the
 // ordered sums' latency) and up to a whole scan.
 template <int CAP, int WARPS, bool SMALL_LIST>
-__global__ void __launch_bounds__(32 * WARPS, SMALL_LIST ? NUSLAM_BIGS_CTAS : 5) k_scan_fit_big(const float * __restrict__ ranges, double min_range, double max_range, ScanPipe pipe)
+__global__ void __launch_bounds__(32 * WARPS, SMALL_LIST ? kBigSmallCtas : 5) k_scan_fit_big(const float * __restrict__ ranges, double min_range, double max_range, ScanPipe pipe)
 {
     __shared__ double zbuf[WARPS][4 * CAP];
     __shared__ double angbuf[WARPS][3 * CAP];
@@ -1113,10 +1105,7 @@ __global__ void k_scan_publish(int64_t chunk, int32_t * __restrict__ n_clusters,
     n_circles[s] = published;
 }
 
-#ifndef NUSLAM_SCAN_CHUNK
-#define NUSLAM_SCAN_CHUNK 262144
-#endif
-constexpr int64_t kScanChunk = NUSLAM_SCAN_CHUNK;   // scans per pipeline pass (bounds the scratch: 262144 x 32 x 60 B = 0.5 GB of the 180 GB; fewer, longer launches: measured best of 64 K / 128 K / 256 K)
+constexpr int64_t kScanChunk = 262144;   // scans per pipeline pass (bounds the scratch: 262144 x 32 x 60 B = 0.5 GB of the 180 GB; fewer, longer launches: measured best of 64 K / 128 K / 256 K)
 
 struct ScanScratch
 {
@@ -1224,7 +1213,7 @@ inline cudaError_t launch_scan_detect(const float * ranges, int64_t n_scans, dou
         if (e != cudaSuccess) return e;
         k_scan_fit_small<kFitSmall, false><<<(unsigned) (sm_count * kFitCtas), kFitThreads, fit_smem16, stream>>>(ranges, min_range, max_range, pipe);
         k_scan_fit_small<kFitNMax, true><<<(unsigned) (sm_count * 3), kFitThreads, fit_smem32, side.s1>>>(ranges, min_range, max_range, pipe);
-        k_scan_fit_big<kFitBigSmall + 2, 4, true><<<(unsigned) (sm_count * NUSLAM_BIGS_CTAS), 128, 0, side.s2>>>(ranges, min_range, max_range, pipe);
+        k_scan_fit_big<kFitBigSmall + 2, 4, true><<<(unsigned) (sm_count * kBigSmallCtas), 128, 0, side.s2>>>(ranges, min_range, max_range, pipe);
         k_scan_fit_big<kBeams + 2, 2, false><<<(unsigned) (sm_count * 5), 64, 0, side.s2>>>(ranges, min_range, max_range, pipe);
         // scans with more than kMaxFastClusters clusters: the one-warp-per-scan kernel over their list (it writes those scans' outputs itself)
         k_scan_detect<true><<<(unsigned) sm_count, 32 * kScanWarps, smem, side.s2>>>(ranges, n_scans, min_range, max_range, cluster_of_beam, n_clusters,

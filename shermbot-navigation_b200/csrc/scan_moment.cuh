@@ -22,15 +22,6 @@
 #include "scan_detect.cuh"
 #include "fastmath.cuh"
 
-#ifdef NUSLAM_SCAN_DEBUG
-#include <cstdio>
-#define NUSLAM_DBG(...) do { if (lane == 0) printf(__VA_ARGS__); } while (0)
-#define NUSLAM_CHK(cond, code) do { if (!(cond)) printf("CHECK %d failed: lane %d\n", code, lane); } while (0)
-#else
-#define NUSLAM_DBG(...)
-#define NUSLAM_CHK(cond, code)
-#endif
-
 namespace nuslam
 {
 
@@ -95,10 +86,8 @@ inline float float_above(double v)
     return f;
 }
 
-#ifndef NUSLAM_MOM_MINBLOCKS
-#define NUSLAM_MOM_MINBLOCKS 8   // resident CTAs per SM the register allocation aims at (8 x 4 warps: 64 registers)
-#endif
-__global__ void __launch_bounds__(32 * kMomWarps, NUSLAM_MOM_MINBLOCKS)
+constexpr int kMomMinBlocks = 8;   // resident CTAs per SM the register allocation aims at (8 x 4 warps: 64 registers)
+__global__ void __launch_bounds__(32 * kMomWarps, kMomMinBlocks)
 k_scan_moment(const float * __restrict__ ranges, const int64_t n_scans, const double min_range, const double max_range, const ScanGate gate,
               int16_t * __restrict__ cluster_of_beam, int32_t * __restrict__ n_clusters, int32_t * __restrict__ n_circles,
               double * __restrict__ circles, const int max_circles, const int scan_ub, int32_t * __restrict__ slow, int32_t * __restrict__ slow_count)
@@ -518,17 +507,13 @@ inline cudaError_t launch_scan_moment(const float * ranges, int64_t n_scans, dou
     gate.max_f = float_below(max_range);
     gate.min_f = float_above(min_range);
     int64_t blocks = (n_scans + kMomWarps - 1) / kMomWarps;
-    const int64_t resident = (int64_t) sm_count * NUSLAM_MOM_MINBLOCKS;
+    const int64_t resident = (int64_t) sm_count * kMomMinBlocks;
     if (blocks > resident) blocks = resident;
     if (blocks < 1) blocks = 1;
     k_scan_moment<<<(unsigned) blocks, 32 * kMomWarps, 0, stream>>>(ranges, n_scans, min_range, max_range, gate, cluster_of_beam, n_clusters, n_circles,
                                                                  circles, max_circles, scan_ub, slow, slow_count);
     e = cudaGetLastError();
     if (e != cudaSuccess) return e;
-#ifdef NUSLAM_SCAN_DEBUG
-    e = cudaStreamSynchronize(stream);
-    fprintf(stderr, "[launch_scan_moment] k_scan_moment done: %s\n", cudaGetErrorString(e));
-#endif
     // the scans the moment route does not decide: oracle-order clustering + Jacobi fit, one warp per scan (usually an empty list)
     const size_t smem = sizeof(ScanSmem) * kScanWarps;
     static bool configured_dev[kMaxDevices] = {false};
