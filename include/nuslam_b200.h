@@ -113,7 +113,15 @@ enum
 {
     NUSLAM_OPT_WRAP_INNOVATION = 1,     /* bearing innovation wrapped to (-pi, pi] in update and associateLandmark (reference: :229-231, :272 do not) */
     NUSLAM_OPT_JOSEPH = 2,              /* Sigma <- (I-KH) Sigma (I-KH)^T + K R K^T, then (Sigma + Sigma^T)/2 (reference: (I-KH) Sigma, :279) */
-    NUSLAM_OPT_PRE_MOTION_JACOBIAN = 4  /* getA evaluated at theta BEFORE the motion update (reference: after it, :129) */
+    NUSLAM_OPT_PRE_MOTION_JACOBIAN = 4, /* getA evaluated at theta BEFORE the motion update (reference: after it, :129) */
+    /* associateLandmark by individual-compatibility nearest neighbour (reference: the FIRST candidate k = 1..seen whose distance
+     * decides wins, :208-249). Every candidate is evaluated; a singular psi at any of them flags NUSLAM_FILTER_SINGULAR and returns
+     * NUSLAM_ID_EXCEPTION. The smallest Mahalanobis distance d* (exact comparison, ties to the lowest id, NaN never a candidate) is a
+     * match when d* < assoc_min (the gate), ambiguous (-1) when d* < assoc_max (the new-landmark threshold), and otherwise opens a
+     * landmark. Only opening one on a full map (seen == n) flags NUSLAM_FILTER_MAP_FULL; a match there succeeds. A chi-square gate
+     * such as 9.21 (99 %, 2 dof) with assoc_max = 60 is the intended use; combine it with NUSLAM_OPT_WRAP_INNOVATION, since an
+     * unwrapped bearing innovation near +-pi defeats any distance rule. */
+    NUSLAM_OPT_NEAREST_NEIGHBOUR = 8
 };
 
 /* Q = 0.1 I, R = 0.001 I (nuslam/config/slam_params.yaml:2-3), thresholds 0.01 / 60, STRICT mode */

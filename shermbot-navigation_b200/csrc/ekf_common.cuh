@@ -23,7 +23,7 @@ constexpr int kStatusSingular = 2;
 constexpr int kStatusBadId = 4;
 constexpr int kIdException = -1000;
 // opt-in departures from the reference: keep in sync with NUSLAM_OPT_* in include/nuslam_b200.h
-constexpr unsigned kOptWrapInnovation = 1u, kOptJoseph = 2u, kOptPreMotionJacobian = 4u;
+constexpr unsigned kOptWrapInnovation = 1u, kOptJoseph = 2u, kOptPreMotionJacobian = 4u, kOptNearestNeighbour = 8u;
 
 // Function attributes and __device__ tables are per DEVICE (per context): one-time setup is remembered per device ordinal, so that
 // a process driving several GPUs (one handle each) configures every one of them. Races between host threads are benign (the setup
@@ -88,6 +88,26 @@ __device__ __forceinline__ bool inv2x2(double p, double q, double r, double s, d
     i10 = div_(-r, det);
     i11 = div_(p, det);
     return true;
+}
+
+// Nearest-neighbour association (NUSLAM_OPT_NEAREST_NEIGHBOUR): candidate (d1, k1) beats (d0, k0) in the lexicographic (d, k) order,
+// an exact fp64 comparison with ties to the lower k. k = 0 is "no candidate" (none yet, or a NaN distance), which anything beats.
+__device__ __forceinline__ bool nn_better(double d1, int k1, double d0, int k0) { return k1 != 0 && (k0 == 0 || d1 < d0 || (d1 == d0 && k1 < k0)); }
+
+// the (d, k) minimum over a full warp by butterfly shuffles: every lane ends with the same winner, whatever order the lanes run in
+__device__ __forceinline__ void nn_warp_min(double & d, int & k)
+{
+#pragma unroll
+    for (int off = kWarp / 2; off > 0; off >>= 1)
+    {
+        const double od = __shfl_xor_sync(0xffffffffu, d, off);
+        const int ok = __shfl_xor_sync(0xffffffffu, k, off);
+        if (nn_better(od, ok, d, k))
+        {
+            d = od;
+            k = ok;
+        }
+    }
 }
 
 }   // namespace nuslam

@@ -494,18 +494,31 @@ __global__ void __launch_bounds__(256) k_large_update(const LargeParams p, const
 // slot the update kernel reads). kind: 0 = inv(psi) throws, 1 = match (d < 0.01), 2 = ambiguous (0.01 < d < 60).
 // single_call: the single associateLandmark call (kOpAssociate) with i_pass = 0 -- it associates whatever the sticky status says.
 // OPT: JOSEPH forms the sub-block as large_update does under it, WRAP wraps the bearing innovation (WarpFilter::mahalanobis).
+// NEAREST_NEIGHBOUR: no key goes to `result`; each CTA reduces its candidates to one exact (d, k, singular) triple in nn[b][blockIdx.x]
+// (no floating-point atomics: the winner does not depend on the order in which CTAs finish) and k_large_assoc_finalize scans them.
+// A full map still evaluates its candidates there: a match succeeds, only a new landmark throws.
+struct LargeNNSlot
+{
+    double d;       // smallest distance of the CTA's candidates
+    int32_t k;      // its candidate (lowest k on ties); 0: none (every distance NaN)
+    int32_t singular;
+};
+
 template <unsigned OPT>
 __global__ void __launch_bounds__(128) k_large_associate(const LargeParams p, const double * __restrict__ z, int m, int i_meas, int i_pass,
                                                          const double * __restrict__ x_cur, const int32_t * __restrict__ seen,
-                                                         int32_t * __restrict__ result, double amin, double amax, bool single_call)
+                                                         int32_t * __restrict__ result, double amin, double amax, bool single_call,
+                                                         LargeNNSlot * __restrict__ nn)
 {
+    constexpr bool kNN = (OPT & kOptNearestNeighbour) != 0;
     const int b = blockIdx.y;
     const int len = p.len;
     const int sn = seen[b];
     if (!single_call && (p.status[b] & (kStatusMapFull | kStatusSingular))) return;   // the reference process died on an earlier measurement
     if (p.m_valid && i_meas >= p.m_valid[b]) return;                 // past this filter's measurement count
     if (p.strict_from && p.strict_from[b] <= i_pass) return;         // this filter's measurements from i_pass on: oracle-order tail
-    if (sn == 0 || 3 + 2 * sn >= len) return;                        // first landmark / full map: decided without any candidate
+    if (sn == 0 || (!kNN && 3 + 2 * sn >= len)) return;              // first landmark / full map: decided without any candidate
+    if (kNN && (int) (blockIdx.x * blockDim.x) >= sn) return;         // a CTA without candidates writes no slot
     const double * S = p.sigma + (int64_t) b * len * len;
     const double * U = p.U + (int64_t) b * 2 * kLargeMMax * len;
     const double * V = p.V + (int64_t) b * 2 * kLargeMMax * len;
@@ -519,8 +532,8 @@ __global__ void __launch_bounds__(128) k_large_associate(const LargeParams p, co
     }
     __syncthreads();
     const int k = blockIdx.x * blockDim.x + threadIdx.x + 1;
-    if (k > sn) return;
-    const int c = 3 + 2 * (k - 1);
+    if (!kNN && k > sn) return;
+    const int c = 3 + 2 * ((kNN && k > sn ? sn : k) - 1);   // NN: every thread takes part in the CTA's reduction (past `seen`: a valid slot, no candidate)
     const int idx[5] = {0, 1, 2, c, c + 1};
     constexpr bool kJoseph = (OPT & kOptJoseph) != 0;
     double B5[5][5];
@@ -577,6 +590,7 @@ __global__ void __launch_bounds__(128) k_large_associate(const LargeParams p, co
     const double det = psi[0][0] * psi[1][1] - psi[0][1] * psi[1][0];
     const double z0 = z[(int64_t) (b * m + i_meas) * 2], z1 = z[(int64_t) (b * m + i_meas) * 2 + 1];
     int kind = -1;
+    double dnn = 0.0;
     if (det == 0.0 || !(fabs(det) < 1.0e300) || !(fabs(1.0 / det) < 1.0e300)) kind = 0;
     else
     {
@@ -586,19 +600,79 @@ __global__ void __launch_bounds__(128) k_large_associate(const LargeParams p, co
         if (OPT & kOptWrapInnovation) dz1 = normalize_angle(dz1);
         const double t0 = dz0 * i00 + dz1 * i10, t1 = dz0 * i01 + dz1 * i11;
         const double d = t0 * dz0 + t1 * dz1;
-        if (d < amin) kind = 1;
+        if (kNN) dnn = d;
+        else if (d < amin) kind = 1;
         else if (d > amin && d < amax) kind = 2;
+    }
+    if (kNN)
+    {
+        const bool active = k <= sn;
+        double d = dnn;
+        int kd = (active && kind != 0 && dnn == dnn) ? k : 0;
+        nn_warp_min(d, kd);
+        const bool sing = __ballot_sync(0xffffffffu, active && kind == 0) != 0u;
+        __shared__ double wd[4];
+        __shared__ int wk[4], ws[4];
+        const int warp = threadIdx.x / kWarp;
+        if (threadIdx.x % kWarp == 0)
+        {
+            wd[warp] = d;
+            wk[warp] = kd;
+            ws[warp] = sing;
+        }
+        __syncthreads();
+        if (threadIdx.x == 0)
+        {
+            int s = ws[0];
+            for (int w = 1; w < 4; ++w)
+            {
+                s |= ws[w];
+                if (nn_better(wd[w], wk[w], d, kd))
+                {
+                    d = wd[w];
+                    kd = wk[w];
+                }
+            }
+            nn[(int64_t) b * gridDim.x + blockIdx.x] = LargeNNSlot{d, kd, s};
+        }
+        return;
     }
     if (kind >= 0) atomicMin(&result[b], (k << 2) | kind);
 }
 
 // slam.cpp:291 for every filter: the id associateLandmark returns, its side effect on `seen`, and the status bits where it throws.
 // ids_slot: B x m scratch the update kernel reads (id <= 0: no update); ids_out: B x m or null.
+// kNN (NUSLAM_OPT_NEAREST_NEIGHBOUR): one warp per filter; the winner is the (d, k) minimum over the ceil(seen / 128) CTA slots
+// k_large_associate wrote (lane s reads slot s: one memory round trip instead of one per slot), and lane 0 decides.
+template <bool kNN>
 __global__ void k_large_assoc_finalize(const LargeParams p, int m, int i_meas, int i_pass, int32_t * __restrict__ seen, int32_t * __restrict__ result,
-                                       int32_t * __restrict__ ids_slot, int32_t * __restrict__ ids_out, bool single_call)
+                                       int32_t * __restrict__ ids_slot, int32_t * __restrict__ ids_out, bool single_call,
+                                       const LargeNNSlot * __restrict__ nn, double amin, double amax)
 {
-    const int b = blockIdx.x * blockDim.x + threadIdx.x;
+    const int b = kNN ? (int) blockIdx.x : (int) (blockIdx.x * blockDim.x + threadIdx.x);
     if (b >= p.batch) return;
+    double dn = 0.0;
+    int kn = 0;
+    bool sing = false;
+    if (kNN)
+    {
+        // (the slots are read whatever the checks below decide; only the branch that follows an associate launch uses them)
+        const int slots = (p.n + 127) / 128, used = (seen[b] + 127) / 128;
+        int sg = 0;
+        for (int s = threadIdx.x; s < used; s += kWarp)   // ascending k within a lane: a later slot wins only with a smaller distance
+        {
+            const LargeNNSlot e = nn[(int64_t) b * slots + s];
+            sg |= e.singular;
+            if (nn_better(e.d, e.k, dn, kn))
+            {
+                dn = e.d;
+                kn = e.k;
+            }
+        }
+        nn_warp_min(dn, kn);
+        sing = __any_sync(0xffffffffu, sg != 0);
+        if (threadIdx.x != 0) return;
+    }
     if (p.m_valid && i_meas >= p.m_valid[b])   // no measurement in this slot (k_large_associate left `result` untouched)
     {
         ids_slot[(int64_t) b * m + i_meas] = 0;
@@ -622,10 +696,30 @@ __global__ void k_large_assoc_finalize(const LargeParams p, int m, int i_meas, i
         id = 1;   // :196-200
         tail = true;
     }
-    else if (3 + 2 * sn >= p.len)
+    else if (!kNN && 3 + 2 * sn >= p.len)
     {
         p.status[b] = st | kStatusMapFull;   // temp(3 + 2 seen) out of bounds: Armadillo throws (:204-207)
         id = kIdException;
+    }
+    else if (kNN)
+    {
+        if (sing)
+        {
+            p.status[b] = st | kStatusSingular;
+            id = kIdException;
+        }
+        else if (kn != 0 && dn < amin) id = kn;
+        else if (kn != 0 && dn < amax) id = -1;
+        else if (3 + 2 * sn >= p.len)   // no slot left for the new landmark
+        {
+            p.status[b] = st | kStatusMapFull;
+            id = kIdException;
+        }
+        else
+        {
+            id = sn + 1;
+            tail = true;
+        }
     }
     else
     {
@@ -711,7 +805,7 @@ __global__ void __launch_bounds__(32) k_large_strict_tail(const LargeParams p, c
     f.len = p.len;
     f.n = p.n;
     f.lane = lane;
-    f.opt = OPT;
+    f.opt = OPT | (p.options & kOptNearestNeighbour);   // the pass's template bits do not carry the association rule
     f.S = p.sigma + (int64_t) b * p.len * p.len;
     f.x = x_cur + (int64_t) b * p.len;
     double * scratch = p.U + (int64_t) b * 2 * kLargeMMax * p.len;
@@ -1186,32 +1280,46 @@ struct LargeAssoc
     int32_t * ids_slot = nullptr;   // B x m
     int32_t * result = nullptr;     // B, initialised to INT_MAX
     int32_t * ids_out = nullptr;    // B x m or null
+    LargeNNSlot * nn = nullptr;     // B x ceil(n / 128) (NUSLAM_OPT_NEAREST_NEIGHBOUR only)
     double amin = 0.01, amax = 60.0;
 };
 
-// k_large_associate for measurement i_meas of the step (slot i_pass of the pass), one thread per candidate landmark
+// k_large_associate for measurement i_meas of the step (slot i_pass of the pass), one thread per candidate landmark, then
+// k_large_assoc_finalize. OPT: the pass's bits (kLargePassOpts); the association rule comes from p.options.
 template <unsigned OPT>
-inline void launch_large_associate_t(const LargeParams & p, const double * z, int m, int i_meas, int i_pass, const double * x_cur, const int32_t * seen,
-                                     int32_t * result, double amin, double amax, bool single_call, cudaStream_t st)
+inline void launch_large_associate_t(const LargeParams & p, const double * z, int m, int i_meas, int i_pass, const double * x_cur, int32_t * seen,
+                                     int32_t * ids_slot, int32_t * ids_out, const LargeAssoc & a, bool single_call, cudaStream_t st)
 {
-    k_large_associate<OPT><<<dim3((unsigned) ((p.n + 127) / 128), (unsigned) p.batch), 128, 0, st>>>(p, z, m, i_meas, i_pass, x_cur, seen, result, amin,
-                                                                                                   amax, single_call);
+    const dim3 grid((unsigned) ((p.n + 127) / 128), (unsigned) p.batch);
+    if (p.options & kOptNearestNeighbour)
+    {
+        k_large_associate<OPT | kOptNearestNeighbour><<<grid, 128, 0, st>>>(p, z, m, i_meas, i_pass, x_cur, seen, a.result, a.amin, a.amax, single_call,
+                                                                          a.nn);
+        k_large_assoc_finalize<true><<<(unsigned) p.batch, kWarp, 0, st>>>(p, m, i_meas, i_pass, seen, a.result, ids_slot, ids_out, single_call, a.nn,
+                                                                            a.amin, a.amax);
+    }
+    else
+    {
+        k_large_associate<OPT><<<grid, 128, 0, st>>>(p, z, m, i_meas, i_pass, x_cur, seen, a.result, a.amin, a.amax, single_call, nullptr);
+        k_large_assoc_finalize<false><<<(unsigned) ((p.batch + 63) / 64), 64, 0, st>>>(p, m, i_meas, i_pass, seen, a.result, ids_slot, ids_out,
+                                                                                        single_call, nullptr, a.amin, a.amax);
+    }
 }
 
-// the option bits the pass kernels take as template arguments (PRE_MOTION_JACOBIAN is predict's alone)
+// the option bits the pass kernels take as template arguments (PRE_MOTION_JACOBIAN is predict's alone, NEAREST_NEIGHBOUR the
+// association's: launch_large_associate_t and k_large_strict_tail read it from p.options)
 constexpr unsigned kLargePassOpts = kOptWrapInnovation | kOptJoseph;
 
-inline void launch_large_associate(const LargeParams & p, const double * z, int m, int i_meas, int i_pass, const double * x_cur, const int32_t * seen,
-                                   int32_t * result, double amin, double amax, bool single_call, cudaStream_t st)
+// the single associateLandmark call: i_pass = 0, no tail
+inline void launch_large_associate(const LargeParams & p, const double * z, int32_t * seen, int32_t * ids_slot, int32_t * id_out, const LargeAssoc & a,
+                                   cudaStream_t st)
 {
     switch (p.options & kLargePassOpts)
     {
-    case 0u: launch_large_associate_t<0u>(p, z, m, i_meas, i_pass, x_cur, seen, result, amin, amax, single_call, st); break;
-    case kOptWrapInnovation:
-        launch_large_associate_t<kOptWrapInnovation>(p, z, m, i_meas, i_pass, x_cur, seen, result, amin, amax, single_call, st);
-        break;
-    case kOptJoseph: launch_large_associate_t<kOptJoseph>(p, z, m, i_meas, i_pass, x_cur, seen, result, amin, amax, single_call, st); break;
-    default: launch_large_associate_t<kLargePassOpts>(p, z, m, i_meas, i_pass, x_cur, seen, result, amin, amax, single_call, st); break;
+    case 0u: launch_large_associate_t<0u>(p, z, 1, 0, 0, p.x, seen, ids_slot, id_out, a, true, st); break;
+    case kOptWrapInnovation: launch_large_associate_t<kOptWrapInnovation>(p, z, 1, 0, 0, p.x, seen, ids_slot, id_out, a, true, st); break;
+    case kOptJoseph: launch_large_associate_t<kOptJoseph>(p, z, 1, 0, 0, p.x, seen, ids_slot, id_out, a, true, st); break;
+    default: launch_large_associate_t<kLargePassOpts>(p, z, 1, 0, 0, p.x, seen, ids_slot, id_out, a, true, st); break;
     }
 }
 
@@ -1242,9 +1350,7 @@ inline cudaError_t launch_large_updates_t(LargeParams & p, const double * z, con
         // unknown correspondence: per measurement associate (one thread per candidate) -> finalize -> update
         for (int k = 0; k < cnt; ++k)
         {
-            launch_large_associate_t<OPT>(p, z, m, i0 + k, k, p.x, seen, assoc->result, assoc->amin, assoc->amax, false, st);
-            k_large_assoc_finalize<<<(unsigned) ((p.batch + 63) / 64), 64, 0, st>>>(p, m, i0 + k, k, seen, assoc->result, assoc->ids_slot, assoc->ids_out,
-                                                                                 false);
+            launch_large_associate_t<OPT>(p, z, m, i0 + k, k, p.x, seen, assoc->ids_slot, assoc->ids_out, *assoc, false, st);
             k_large_update<OPT><<<grid, threads, 0, st>>>(p, z + 2 * (int64_t) i0, assoc->ids_slot + i0, m, k, p.x, p.x2, seen_snapshot, seen);
             double * tmp = p.x;
             p.x = p.x2;

@@ -221,6 +221,7 @@ struct WarpFilter
             seen = 1;
             return 1;
         }
+        if (opt & kOptNearestNeighbour) return associate_nn(z0, z1, seen, status, R, amin, amax);
         if (3 + 2 * seen >= len)   // temp(3+2*seen) out of bounds: Armadillo throws (:206)
         {
             status |= kStatusMapFull;
@@ -248,6 +249,43 @@ struct WarpFilter
                 if ((hitA >> first) & 1u) return base + first + 1;
                 return -1;
             }
+        }
+        seen += 1;
+        return seen;
+    }
+
+    // NUSLAM_OPT_NEAREST_NEIGHBOUR (seen >= 1): every candidate k = 1..seen is evaluated; a singular psi anywhere throws, as the
+    // reference's inv would once it reached that candidate. The smallest distance (lowest k on ties; a NaN distance is no candidate)
+    // is a match below amin, ambiguous below amax, and otherwise the measurement opens a landmark -- which throws on a full map,
+    // where a match still succeeds. Each lane keeps its running minimum over the chunks of 32, then one warp-wide (d, k) reduction.
+    __device__ int associate_nn(double z0, double z1, int & seen, int & status, const double * R, double amin, double amax)
+    {
+        double best = 0.0;
+        int kbest = 0;
+        for (int base = 0; base < seen; base += kWarp)
+        {
+            const int k = base + lane + 1;
+            bool singular = false;
+            double d = 0.0;
+            if (k <= seen) d = mahalanobis(z0, z1, k, R, singular);
+            if (__ballot_sync(0xffffffffu, singular))
+            {
+                status |= kStatusSingular;
+                return kIdException;
+            }
+            if (k <= seen && d == d && nn_better(d, k, best, kbest))
+            {
+                best = d;
+                kbest = k;
+            }
+        }
+        nn_warp_min(best, kbest);
+        if (kbest != 0 && best < amin) return kbest;
+        if (kbest != 0 && best < amax) return -1;
+        if (3 + 2 * seen >= len)   // no slot left for the new landmark
+        {
+            status |= kStatusMapFull;
+            return kIdException;
         }
         seen += 1;
         return seen;

@@ -113,6 +113,7 @@ struct nuslam_ekf
     double * lg_P = nullptr;
     int32_t * lg_seen_snap = nullptr;
     DevBuf lg_ids_slot, lg_assoc_result;   // unknown correspondence in large-map mode
+    DevBuf lg_nn_slots;                    // NUSLAM_OPT_NEAREST_NEIGHBOUR in large-map mode: B x ceil(n / 128) CTA minima
     double * x_snap_next = nullptr;        // pipelined host path: where the next step's kernels also write the state vector
     int32_t * worklist = nullptr;   // batch entries
     int32_t * wl_count = nullptr;   // [0] = entries, [1] = finished blocks of the list kernel, [2] finished warps of the FAST kernel, [3] device-launch error
@@ -263,6 +264,21 @@ nuslam::LargeParams make_large_params(nuslam_ekf * h)
     return p;
 }
 
+// LARGE-MAP mode, unknown correspondence: the association scratch (allocated on first use) and thresholds of `a`
+int large_assoc_scratch(nuslam_ekf * h, nuslam::LargeAssoc & a)
+{
+    int rc = h->lg_assoc_result.reserve(sizeof(int32_t) * h->batch);
+    if (!rc && (h->cfg.options & NUSLAM_OPT_NEAREST_NEIGHBOUR))
+        rc = h->lg_nn_slots.reserve(sizeof(nuslam::LargeNNSlot) * h->batch * ((h->cfg.n_landmarks + 127) / 128));
+    if (rc) return rc;
+    a.result = static_cast<int32_t *>(h->lg_assoc_result.p);
+    a.nn = static_cast<nuslam::LargeNNSlot *>(h->lg_nn_slots.p);
+    a.amin = h->cfg.assoc_min;
+    a.amax = h->cfg.assoc_max;
+    CU(cudaMemsetAsync(a.result, 0x7f, sizeof(int32_t) * h->batch, h->stream));   // any value >= every key; finalize resets to INT_MAX
+    return NUSLAM_OK;
+}
+
 // LARGE-MAP mode: m measurements in delayed passes of at most kLargeMMax; `step_protocol` adds slam.cpp:295-297
 // (initializeLandmark for ids above the scan's seen snapshot, seen = max(seen, id)). m_valid (B or null, unknown correspondence
 // only): filter b uses only its first m_valid[b] measurements; the passes stay planned from m, so the step needs no host read.
@@ -276,14 +292,10 @@ int large_updates(nuslam_ekf * h, const double * z, const int32_t * ids, int m, 
     {
         // unknown correspondence: associateLandmark per measurement against the pass's current covariance
         int rc = h->lg_ids_slot.reserve(sizeof(int32_t) * h->batch * (m > 0 ? m : 1));
-        if (!rc) rc = h->lg_assoc_result.reserve(sizeof(int32_t) * h->batch);
+        if (!rc) rc = large_assoc_scratch(h, assoc);
         if (rc) return rc;
         assoc.ids_slot = static_cast<int32_t *>(h->lg_ids_slot.p);
-        assoc.result = static_cast<int32_t *>(h->lg_assoc_result.p);
         assoc.ids_out = ids_out;
-        assoc.amin = h->cfg.assoc_min;
-        assoc.amax = h->cfg.assoc_max;
-        CU(cudaMemsetAsync(assoc.result, 0x7f, sizeof(int32_t) * h->batch, h->stream));   // any value >= every key; finalize resets to INT_MAX
         // slots no kernel writes read 0: those a filter's oracle-order tail never reaches (past its count, or after its process died)
         if (ids_out && m > 0) CU(cudaMemsetAsync(ids_out, 0, sizeof(int32_t) * h->batch * m, h->stream));
     }
@@ -306,15 +318,11 @@ int large_associate(nuslam_ekf * h, const double * z, int32_t * id_out)
 {
     nuslam::LargeParams p = make_large_params(h);
     p.strict_from = nullptr;
+    nuslam::LargeAssoc assoc;
     int rc = h->lg_ids_slot.reserve(sizeof(int32_t) * h->batch);
-    if (!rc) rc = h->lg_assoc_result.reserve(sizeof(int32_t) * h->batch);
+    if (!rc) rc = large_assoc_scratch(h, assoc);
     if (rc) return rc;
-    int32_t * result = static_cast<int32_t *>(h->lg_assoc_result.p);
-    CU(cudaMemsetAsync(result, 0x7f, sizeof(int32_t) * h->batch, h->stream));
-    nuslam::launch_large_associate(p, z, 1, 0, 0, h->x, h->seen, result, h->cfg.assoc_min, h->cfg.assoc_max, true, h->stream);
-    CU(cudaGetLastError());
-    nuslam::k_large_assoc_finalize<<<(unsigned) ((p.batch + 63) / 64), 64, 0, h->stream>>>(p, 1, 0, 0, h->seen, result,
-                                                                                          static_cast<int32_t *>(h->lg_ids_slot.p), id_out, true);
+    nuslam::launch_large_associate(p, z, h->seen, static_cast<int32_t *>(h->lg_ids_slot.p), id_out, assoc, h->stream);
     CU(cudaGetLastError());
     return NUSLAM_OK;
 }
@@ -351,7 +359,8 @@ int nuslam_ekf_create(const nuslam_ekf_config * cfg, int64_t batch, int device, 
     if (!cfg || !out) return fail(NUSLAM_ERR_INVALID, "null config or output pointer");
     if (cfg->n_landmarks < 1 || batch < 1) return fail(NUSLAM_ERR_INVALID, "n_landmarks and batch must be >= 1");
     if (cfg->mode != NUSLAM_MODE_STRICT && cfg->mode != NUSLAM_MODE_FAST && cfg->mode != NUSLAM_MODE_LARGE) return fail(NUSLAM_ERR_INVALID, "unknown mode");
-    if (cfg->options & ~(uint32_t) (NUSLAM_OPT_WRAP_INNOVATION | NUSLAM_OPT_JOSEPH | NUSLAM_OPT_PRE_MOTION_JACOBIAN)) return fail(NUSLAM_ERR_INVALID, "unknown option bit");
+    if (cfg->options & ~(uint32_t) (NUSLAM_OPT_WRAP_INNOVATION | NUSLAM_OPT_JOSEPH | NUSLAM_OPT_PRE_MOTION_JACOBIAN | NUSLAM_OPT_NEAREST_NEIGHBOUR))
+        return fail(NUSLAM_ERR_INVALID, "unknown option bit");
     if (!(cfg->landmark_prior > 0.0)) return fail(NUSLAM_ERR_INVALID, "landmark_prior must be positive (default config sets INT_MAX)");
     int ndev = 0;
     cudaError_t e = cudaGetDeviceCount(&ndev);
@@ -459,6 +468,7 @@ int nuslam_ekf_destroy(nuslam_ekf * h)
     if (h->lg_seen_snap) cudaFree(h->lg_seen_snap);
     h->lg_ids_slot.release();
     h->lg_assoc_result.release();
+    h->lg_nn_slots.release();
     if (h->worklist) cudaFree(h->worklist);
     if (h->wl_count) cudaFree(h->wl_count);
     h->s_tw.release();

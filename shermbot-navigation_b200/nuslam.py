@@ -42,6 +42,11 @@ EXPORTS = [
 
 
 OPT_WRAP_INNOVATION, OPT_JOSEPH, OPT_PRE_MOTION_JACOBIAN = 1, 2, 4   # include/nuslam_b200.h NUSLAM_OPT_*
+# associateLandmark by nearest neighbour instead of the reference's first deciding candidate: the closest candidate matches when its
+# Mahalanobis distance is below assoc_min (the gate, e.g. 9.21), is ambiguous (-1) below assoc_max (the new-landmark threshold, e.g.
+# 60), and otherwise opens a landmark. Combine it with OPT_WRAP_INNOVATION: an unwrapped bearing innovation near +-pi defeats any
+# distance rule.
+OPT_NEAREST_NEIGHBOUR = 8
 
 
 class NuslamError(RuntimeError):
@@ -137,7 +142,10 @@ def _mem_of(*ptrs):
 
 
 class BatchedExtendedKalman:
-    """B independent ``slam_library::ExtendedKalman`` filters on one B200."""
+    """B independent ``slam_library::ExtendedKalman`` filters on one B200.
+
+    ``assoc_min`` / ``assoc_max`` are associateLandmark's thresholds (0.01 / 60 in the reference). Under ``options`` with
+    OPT_NEAREST_NEIGHBOUR, ``assoc_min`` is the gate of the nearest candidate and ``assoc_max`` the new-landmark threshold."""
 
     def __init__(self, robotState, mapState=None, Q=None, R=None, n_landmarks=None, mode="strict", device=0,
                  stream=None, assoc_min=0.01, assoc_max=60.0, options=0, landmark_prior=None):
