@@ -85,7 +85,10 @@ enum
     NUSLAM_FILTER_MAP_FULL = 1,   /* associateLandmark with seen == n: Armadillo bounds check throws (slam_library.cpp:206).
                                      The filter is frozen from that measurement on, as the reference process would be dead. */
     NUSLAM_FILTER_SINGULAR = 2,   /* det(H Sigma H^T + R) == 0: arma::inv throws (slam_library.cpp:231,270); update skipped */
-    NUSLAM_FILTER_BAD_ID = 4      /* update/initializeLandmark with id outside 1..n: bounds check throws; call skipped */
+    NUSLAM_FILTER_BAD_ID = 4,     /* update/initializeLandmark with id outside 1..n: bounds check throws; call skipped */
+    NUSLAM_FILTER_ASSOC_TRUNCATED = 8 /* NUSLAM_OPT_JOINT_COMPATIBILITY: a step's search hit its budget of joint tests and used the best
+                                         hypothesis found so far. Informational: it never freezes a filter (nuslam_ekf_error_stats
+                                         slot [6] counts such filters too, as it counts any non-zero status). */
 };
 
 /* id written by nuslam_ekf_associate / nuslam_ekf_step where the reference throws */
@@ -121,7 +124,31 @@ enum
      * landmark. Only opening one on a full map (seen == n) flags NUSLAM_FILTER_MAP_FULL; a match there succeeds. A chi-square gate
      * such as 9.21 (99 %, 2 dof) with assoc_max = 60 is the intended use; combine it with NUSLAM_OPT_WRAP_INNOVATION, since an
      * unwrapped bearing innovation near +-pi defeats any distance rule. */
-    NUSLAM_OPT_NEAREST_NEIGHBOUR = 8
+    NUSLAM_OPT_NEAREST_NEIGHBOUR = 8,
+    /* The step's measurements associated jointly: joint compatibility branch and bound (JCBB; Neira & Tardos, IEEE T-RO 2001), in
+     * the oracle-order kernels only (nuslam_ekf_create refuses it with NUSLAM_OPT_NEAREST_NEIGHBOUR or a non-finite or non-positive
+     * assoc_min: NUSLAM_ERR_INVALID; on a large-map handle: NUSLAM_ERR_UNSUPPORTED). assoc_min is the individual gate, a chi-square
+     * value at 2 dof (e.g. 9.21); it fixes conf = 1 - exp(-assoc_min / 2), and p pairings pass jointly when their stacked innovation
+     * has D^2 = nu^T S^-1 nu < T_p = chi2_{2p}^-1(conf) (T_1 = assoc_min), S = H Sigma H^T + blockdiag(R). A step with unknown ids
+     * (nuslam_ekf_step with ids == NULL, nuslam_ekf_scan_step, the step_async paths) takes at most 16 measurements
+     * (NUSLAM_ERR_UNSUPPORTED above) and, after predict:
+     *  1. d_ik, the nearest-neighbour distance, at the predicted state for every measurement i and candidate k = 1..seen; k is
+     *     compatible with i when d_ik < assoc_min (NaN never). A singular psi anywhere flags NUSLAM_FILTER_SINGULAR: the first
+     *     measurement gets NUSLAM_ID_EXCEPTION, the others 0, and no update is applied.
+     *  2. Depth-first search over the measurements in order: measurement i tries its compatible candidates in ascending (d_ik, k),
+     *     skipping landmarks the hypothesis already uses, then no pairing. A pairing is accepted when the joint D^2 of the hypothesis
+     *     it extends (at the predicted Sigma) is < T_p; the first pairing's D^2 is its d_ik, and a child whose S is not positive
+     *     definite is not accepted. A node is pruned when its pairings plus the measurements it has not decided are fewer than the
+     *     best hypothesis' pairings. Better: more pairings, or as many and a strictly smaller D^2. At most 4 096 joint tests per
+     *     filter and step: then the best hypothesis so far is used and NUSLAM_FILTER_ASSOC_TRUNCATED is set.
+     *  3. A paired measurement gets its landmark's id; an unpaired one -1 when some d_ik < assoc_max (the new-landmark threshold),
+     *     otherwise it opens a landmark (seen + 1, seen + 2, ... in measurement order; NUSLAM_FILTER_MAP_FULL and
+     *     NUSLAM_ID_EXCEPTION on a full map, as under NUSLAM_OPT_NEAREST_NEIGHBOUR).
+     *  4. The ids are applied as every step applies associateLandmark's, one sequential update after another.
+     * With one measurement this is nearest neighbour: steps with m = 1 give the bits of a NUSLAM_OPT_NEAREST_NEIGHBOUR handle, and
+     * nuslam_ekf_associate (one measurement per call) runs nearest neighbour. Association sees the predicted map only, so two
+     * measurements of one unseen landmark in a scan open two landmarks. */
+    NUSLAM_OPT_JOINT_COMPATIBILITY = 32
 };
 
 /* Q = 0.1 I, R = 0.001 I (nuslam/config/slam_params.yaml:2-3), thresholds 0.01 / 60, STRICT mode */

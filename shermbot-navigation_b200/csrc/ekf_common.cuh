@@ -21,9 +21,11 @@ constexpr double kFirstTouchVariance = 1.0e6;
 constexpr int kStatusMapFull = 1;
 constexpr int kStatusSingular = 2;
 constexpr int kStatusBadId = 4;
+constexpr int kStatusAssocTruncated = 8;
 constexpr int kIdException = -1000;
 // opt-in departures from the reference: keep in sync with NUSLAM_OPT_* in include/nuslam_b200.h
 constexpr unsigned kOptWrapInnovation = 1u, kOptJoseph = 2u, kOptPreMotionJacobian = 4u, kOptNearestNeighbour = 8u;
+constexpr unsigned kOptJointCompatibility = 32u;
 
 // Function attributes and __device__ tables are per DEVICE (per context): one-time setup is remembered per device ordinal, so that
 // a process driving several GPUs (one handle each) configures every one of them. Races between host threads are benign (the setup

@@ -464,13 +464,340 @@ struct WarpFilter
     }
 };
 
+// NUSLAM_OPT_JOINT_COMPATIBILITY (joint compatibility branch and bound, Neira & Tardos 2001): measurements per step, and joint tests
+// per filter per step before the search stops with the best hypothesis found so far (NUSLAM_FILTER_ASSOC_TRUNCATED)
+constexpr int kJcbbMMax = 16;
+constexpr int kJcbbMaxTests = 4096;
+constexpr int kJcbbRows = 2 * kJcbbMMax;
+
+// JCBB scratch of one warp, behind its WarpFilter slice (JOINT handles only), in doubles
+__host__ __device__ constexpr int jcbb_smem_doubles(int n)
+{
+    return kJcbbMMax * n + 10 * n + kJcbbRows * (kJcbbRows + 1) / 2 + kJcbbRows + 4 * kJcbbMMax + (kJcbbMMax + 1)
+         + (kJcbbMMax * n + 6 * kJcbbMMax + 2 * (kJcbbMMax + 1) + 1) / 2;
+}
+
+struct JcbbScratch
+{
+    double * dist;   // m x n: d_ik, the individual distance of measurement i to candidate k (dist[i * n + k - 1])
+    double * hc;     // n x 10: H entries (h01 h02 h0c h0c1 h11 h12 h1c h1c1), z_hat (range, bearing) of every candidate
+    double * L;      // packed lower Cholesky factor of the hypothesis' joint S, row r at r (r + 1) / 2
+    double * y;      // L^-1 nu, the whitened stacked innovation
+    double * bx;     // per test: 2 x 2 cross blocks H_new Sigma H_j^T of the pairings j < p, then H_new Sigma H_new^T + R at j = p
+    double * d2;     // per depth: D^2 of the hypothesis on entry
+    int * cand;      // m x n: the compatible candidates of measurement i in ascending (d_ik, k)
+    int * ncand;     // m
+    int * jid;       // m: the ids the step applies
+    int * hyp;       // per depth: the landmark measurement i is paired with (0: none)
+    int * best;      // m: the best hypothesis
+    int * pk;        // per pairing: its landmark
+    int * it;        // per depth: next position in cand (ncand: the null pairing, ncand + 1: exhausted)
+    int * pcnt;      // per depth: pairings on entry
+
+    __device__ __forceinline__ void carve(double * base, int n)
+    {
+        dist = base;
+        hc = dist + kJcbbMMax * n;
+        L = hc + 10 * n;
+        y = L + kJcbbRows * (kJcbbRows + 1) / 2;
+        bx = y + kJcbbRows;
+        d2 = bx + 4 * kJcbbMMax;
+        cand = reinterpret_cast<int *>(d2 + kJcbbMMax + 1);
+        ncand = cand + kJcbbMMax * n;
+        jid = ncand + kJcbbMMax;
+        hyp = jid + kJcbbMMax;
+        best = hyp + kJcbbMMax;
+        pk = best + kJcbbMMax;
+        it = pk + kJcbbMMax;
+        pcnt = it + kJcbbMMax + 1;
+    }
+};
+
+// One joint test: D^2 of the hypothesis (pairings pk[0..p), D^2 = d2) extended by measurement (z0, z1) paired with landmark k, whose
+// individual distance is dik. Appends rows 2p, 2p + 1 to L and y (a sibling overwrites them). The joint S is H Sigma H^T + blockdiag(R)
+// at the predicted Sigma; a child whose S is not positive definite comes out NaN or infinite, so it is never accepted. The first
+// pairing's D^2 is its individual distance, the same arithmetic as nearest neighbour. Lanes j < p form the cross blocks, lane p the
+// diagonal block; lanes 0 and 1 solve L l = cross^T for the two new rows; every lane then forms the same 2 x 2 Schur complement.
+__device__ inline double jcbb_joint_test(WarpFilter & f, JcbbScratch & w, double z0, double z1, int k, int p, double dik, double d2,
+                                  const double * R)
+{
+    const int lane = f.lane, len = f.len;
+    const double * hq = w.hc + 10 * (k - 1);
+    const int cq = 3 + 2 * (k - 1);
+    if (lane <= p)
+    {
+        const int kj = lane < p ? w.pk[lane] : k;
+        const double * hj = w.hc + 10 * (kj - 1);
+        const int cj = 3 + 2 * (kj - 1);
+        const int cols[5] = {0, 1, 2, cj, cj + 1};
+        const double hj0[5] = {0.0, hj[0], hj[1], hj[2], hj[3]}, hj1[5] = {-1.0, hj[4], hj[5], hj[6], hj[7]};
+        double b00 = 0.0, b01 = 0.0, b10 = 0.0, b11 = 0.0;
+#pragma unroll
+        for (int t = 0; t < 5; ++t)
+        {
+            const double * col = f.S + cols[t] * len;
+            const double g0 = hq[0] * col[1] + hq[1] * col[2] + hq[2] * col[cq] + hq[3] * col[cq + 1];
+            const double g1 = -col[0] + hq[4] * col[1] + hq[5] * col[2] + hq[6] * col[cq] + hq[7] * col[cq + 1];
+            b00 += g0 * hj0[t];
+            b01 += g0 * hj1[t];
+            b10 += g1 * hj0[t];
+            b11 += g1 * hj1[t];
+        }
+        if (lane == p)
+        {
+            b00 += R[0];
+            b10 += R[1];
+            b01 += R[2];
+            b11 += R[3];
+        }
+        double * o = w.bx + 4 * lane;   // [a * 2 + b] = (H_new Sigma H_j^T)(a, b)
+        o[0] = b00;
+        o[1] = b01;
+        o[2] = b10;
+        o[3] = b11;
+    }
+    __syncwarp();
+    const int P = 2 * p;
+    double * l0 = w.L + P * (P + 1) / 2;
+    double * l1 = l0 + P + 1;
+    if (lane < 2)
+    {
+        double * lr = lane ? l1 : l0;
+        for (int r = 0; r < P; ++r)
+        {
+            const double * Lr = w.L + r * (r + 1) / 2;
+            double v = w.bx[4 * (r >> 1) + 2 * lane + (r & 1)];
+            for (int s = 0; s < r; ++s) v -= Lr[s] * lr[s];
+            lr[r] = v / Lr[r];
+        }
+    }
+    __syncwarp();
+    double s00 = w.bx[4 * p], s10 = w.bx[4 * p + 2], s11 = w.bx[4 * p + 3];
+    double n1 = z1 - hq[9];
+    if (f.opt & kOptWrapInnovation) n1 = normalize_angle(n1);
+    double n0 = z0 - hq[8];
+    for (int r = 0; r < P; ++r)
+    {
+        s00 -= l0[r] * l0[r];
+        s10 -= l1[r] * l0[r];
+        s11 -= l1[r] * l1[r];
+        n0 -= l0[r] * w.y[r];
+        n1 -= l1[r] * w.y[r];
+    }
+    const double a = sqrt(s00), b = s10 / a, e = sqrt(s11 - b * b);
+    const double y0 = n0 / a, y1 = (n1 - b * y0) / e;
+    __syncwarp();
+    if (lane == 0)
+    {
+        l0[P] = a;
+        l1[P] = b;
+        l1[P + 1] = e;
+        w.y[P] = y0;
+        w.y[P + 1] = y1;
+    }
+    __syncwarp();
+    return p == 0 ? dik : d2 + y0 * y0 + y1 * y1;
+}
+
+// NUSLAM_OPT_JOINT_COMPATIBILITY: the ids of one step's measurements z[0..mv) (mv <= kJcbbMMax) at the predicted state, into w.jid;
+// seen and status as the per-measurement rule would leave them. T[p]: the joint threshold of p pairings (T[1] = amin).
+__device__ inline void jcbb_associate(WarpFilter & f, JcbbScratch & w, const double * z, int mv, int & seen, int & status, const double * R,
+                               double amin, double amax, const double * T)
+{
+    const int lane = f.lane, n = f.n, seen0 = seen;
+    // individual phase: every (measurement, candidate) pair, spread over the lanes
+    for (int k = lane + 1; k <= seen0; k += kWarp)
+    {
+        HEntries H;
+        double zr, zb;
+        measurement_model(f.x, 3 + 2 * (k - 1), H, zr, zb);
+        double * h = w.hc + 10 * (k - 1);
+        h[0] = H.h01;
+        h[1] = H.h02;
+        h[2] = H.h0c;
+        h[3] = H.h0c1;
+        h[4] = H.h11;
+        h[5] = H.h12;
+        h[6] = H.h1c;
+        h[7] = H.h1c1;
+        h[8] = zr;
+        h[9] = zb;
+    }
+    bool singular = false;
+    for (int e = lane; e < mv * seen0; e += kWarp)
+    {
+        const int i = e / seen0, k = e - i * seen0 + 1;
+        bool s = false;
+        const double d = f.mahalanobis(z[2 * i], z[2 * i + 1], k, R, s);
+        singular |= s;
+        w.dist[i * n + k - 1] = d;
+    }
+    if (__any_sync(0xffffffffu, singular))
+    {
+        // psi does not depend on the measurement: every measurement has the singular candidate, so the first one throws
+        status |= kStatusSingular;
+        if (lane == 0) w.jid[0] = kIdException;
+        __syncwarp();
+        return;
+    }
+    __syncwarp();
+    for (int e = lane; e < mv * seen0; e += kWarp)
+    {
+        const int i = e / seen0, k = e - i * seen0 + 1;
+        const double * di = w.dist + i * n;
+        const double d = di[k - 1];
+        if (d < amin)
+        {
+            int r = 0;
+            for (int k2 = 1; k2 <= seen0; ++k2)
+            {
+                const double d2 = di[k2 - 1];
+                r += (d2 < amin) && (d2 < d || (d2 == d && k2 < k));
+            }
+            w.cand[i * n + r] = k;
+        }
+    }
+    if (lane < mv)
+    {
+        int c = 0;
+        for (int k = 1; k <= seen0; ++k) c += w.dist[lane * n + k - 1] < amin;
+        w.ncand[lane] = c;
+        w.best[lane] = 0;
+    }
+    __syncwarp();
+
+    // depth-first search over the measurements; every lane runs the same control flow on the same values
+    int tests = 0, best_p = 0;
+    double best_d2 = 0.0;
+    int i = 0, p = 0;
+    double d2 = 0.0;
+    bool entered = true, running = mv > 0 && seen0 > 0;
+    while (running)
+    {
+        if (entered)
+        {
+            entered = false;
+            if (i < mv && p + (mv - i) >= best_p)
+            {
+                __syncwarp();
+                if (lane == 0)
+                {
+                    w.it[i] = 0;
+                    w.pcnt[i] = p;
+                    w.d2[i] = d2;
+                }
+                __syncwarp();
+                continue;
+            }
+            if (i == mv && (p > best_p || (p == best_p && d2 < best_d2)))
+            {
+                best_p = p;
+                best_d2 = d2;
+                __syncwarp();
+                if (lane < mv) w.best[lane] = w.hyp[lane];
+                __syncwarp();
+            }
+            --i;   // pruned, or a leaf: back to the parent's next option
+            p = w.pcnt[i];
+            d2 = w.d2[i];
+            continue;
+        }
+        // node i: its next option
+        const int nc = w.ncand[i];
+        int pos = w.it[i], k = -1;
+        double nd2 = d2;
+        while (pos < nc)
+        {
+            const int kk = w.cand[i * n + pos];
+            ++pos;
+            bool used = false;
+            for (int j = 0; j < p; ++j) used |= w.pk[j] == kk;
+            if (used) continue;
+            if (tests == kJcbbMaxTests)
+            {
+                status |= kStatusAssocTruncated;
+                running = false;
+                break;
+            }
+            ++tests;
+            const double t = jcbb_joint_test(f, w, z[2 * i], z[2 * i + 1], kk, p, w.dist[i * n + kk - 1], d2, R);
+            if (t < T[p + 1])
+            {
+                k = kk;
+                nd2 = t;
+                break;
+            }
+        }
+        if (!running) break;
+        if (k < 0 && pos == nc)   // the null pairing, last
+        {
+            pos = nc + 1;
+            k = 0;
+        }
+        __syncwarp();
+        if (lane == 0)
+        {
+            w.it[i] = pos;
+            if (k >= 0) w.hyp[i] = k;
+            if (k > 0) w.pk[p] = k;
+        }
+        __syncwarp();
+        if (k >= 0)
+        {
+            if (k > 0)
+            {
+                ++p;
+                d2 = nd2;
+            }
+            ++i;
+            entered = true;
+        }
+        else if (i == 0)
+            running = false;
+        else
+        {
+            --i;
+            p = w.pcnt[i];
+            d2 = w.d2[i];
+        }
+    }
+
+    // outcome: the best hypothesis' pairings; an unpaired measurement is ambiguous when any candidate lies below amax, and otherwise
+    // opens a landmark in measurement order (an exception on a full map, and nothing after it)
+    bool full = false;
+    for (int r = 0; r < mv; ++r)
+    {
+        int id = 0;
+        if (!full)
+        {
+            id = w.best[r];
+            if (id == 0)
+            {
+                bool amb = false;
+                for (int k = 1; k <= seen0; ++k) amb |= w.dist[r * n + k - 1] < amax;
+                if (amb) id = -1;
+                else if (seen >= n)
+                {
+                    status |= kStatusMapFull;
+                    full = true;
+                    id = kIdException;
+                }
+                else id = ++seen;
+            }
+        }
+        if (lane == 0) w.jid[r] = id;
+    }
+    __syncwarp();
+}
+
 enum EkfOp
 {
     kOpPredict = 0,
     kOpUpdate = 1,
     kOpAssociate = 2,
     kOpInit = 3,
-    kOpStep = 4
+    kOpStep = 4,
+    kOpStepJoint = 5   // kOpStep with NUSLAM_OPT_JOINT_COMPATIBILITY and unknown ids
 };
 
 struct EkfParams
@@ -493,7 +820,15 @@ struct EkfParams
     double amin, amax;
     // launch shape of k_ekf_strict_list for the filters a FAST kernel hands over (strict_tail below); tail_blocks == 0: the host launches it
     int tail_blocks, tail_threads, tail_smem;
+    const double * joint_t;  // NUSLAM_OPT_JOINT_COMPATIBILITY: the joint thresholds T[p] of p = 1..kJcbbMMax pairings, or null
 };
+
+// per-warp shared memory of the oracle-order kernels, in doubles: the filter, plus the JCBB scratch in the JOINT step
+template <int OP>
+__host__ __device__ constexpr int strict_warp_doubles(int len, int n)
+{
+    return OP == kOpStepJoint ? strict_smem_doubles(len) + jcbb_smem_doubles(n) : strict_smem_doubles(len);
+}
 
 // One warp replays reference call OP on filter b; Sigma staged through the warp's slice of shared memory.
 template <int OP>
@@ -543,7 +878,7 @@ __device__ __forceinline__ void strict_filter(const EkfParams & p, const int64_t
             p.status[b] = status;
         }
     }
-    else if (OP == kOpStep)
+    else if (OP == kOpStep || OP == kOpStepJoint)
     {
         // EKFSlam::main_loop, nuslam/src/slam.cpp:262-319
         const int64_t mb = b * p.m;
@@ -560,6 +895,13 @@ __device__ __forceinline__ void strict_filter(const EkfParams & p, const int64_t
         const int mv = p.m_valid ? min(p.m, max(0, p.m_valid[b])) : p.m;   // markers this filter received (landmarks.cpp:84-109)
         if (p.ids_out)
             for (int i = mv + lane; i < p.m; i += kWarp) p.ids_out[mb + i] = 0;
+        JcbbScratch jw;
+        if (OP == kOpStepJoint)
+        {
+            // every measurement's id at once (the predicted state); the loop below applies them as it would apply associate's
+            jw.carve(smem_warp + strict_smem_doubles(p.len), p.n);
+            jcbb_associate(f, jw, p.z + 2 * mb, mv, seen, status, p.R, p.amin, p.amax, p.joint_t);
+        }
         for (int i = 0; i < mv; ++i)                                  // slam.cpp:279
         {
             const double z0 = p.z[2 * (mb + i)], z1 = p.z[2 * (mb + i) + 1];
@@ -584,7 +926,8 @@ __device__ __forceinline__ void strict_filter(const EkfParams & p, const int64_t
             }
             else
             {
-                id = f.associate(z0, z1, seen, status, p.R, p.amin, p.amax);   // slam.cpp:291
+                if (OP == kOpStepJoint) id = jw.jid[i];
+                else id = f.associate(z0, z1, seen, status, p.R, p.amin, p.amax);   // slam.cpp:291
                 if (id == kIdException)
                 {
                     if (p.ids_out)
@@ -616,7 +959,7 @@ __global__ void __launch_bounds__(128) k_ekf_strict(const EkfParams p)
     const int warp = threadIdx.x / kWarp, lane = threadIdx.x % kWarp;
     const int64_t b = (int64_t) blockIdx.x * (blockDim.x / kWarp) + warp;
     if (b >= p.batch) return;
-    strict_filter<OP>(p, b, smem + (size_t) warp * strict_smem_doubles(p.len), lane);
+    strict_filter<OP>(p, b, smem + (size_t) warp * strict_warp_doubles<OP>(p.len, p.n), lane);
 }
 
 // One warp per filter over a device-side work list (the filters the FAST kernel handed over because their step

@@ -4,6 +4,7 @@
 // launches the kernels in ekf_strict.cuh / ekf_fast.cuh / scan_detect.cuh. No CPU arithmetic path exists
 // here: without a CUDA device every compute entry point fails with NUSLAM_ERR_CUDA.
 #include <cuda_runtime.h>
+#include <math.h>
 #include <stdint.h>
 #include <stdio.h>
 #include <string.h>
@@ -119,6 +120,7 @@ struct nuslam_ekf
     int32_t * wl_count = nullptr;   // [0] = entries, [1] = finished blocks of the list kernel, [2] finished warps of the FAST kernel, [3] device-launch error
     size_t strict_smem = 0;   // per-warp shared memory of the strict kernels, bytes
     int strict_warps = 4;
+    DevBuf joint_t;           // NUSLAM_OPT_JOINT_COMPATIBILITY: T[0..kJcbbMMax], the joint thresholds
 };
 
 namespace
@@ -169,7 +171,47 @@ nuslam::EkfParams make_params(nuslam_ekf * h)
     p.amax = h->cfg.assoc_max;
     p.options = h->cfg.options;
     p.x_snap = h->x_snap_next;
+    p.joint_t = static_cast<const double *>(h->joint_t.p);
     return p;
+}
+
+// NUSLAM_OPT_JOINT_COMPATIBILITY: T[p] = chi2_{2p}^-1(conf), conf = 1 - exp(-amin / 2), so T[1] = amin. Bisection on the survival function
+// of chi2 at even degrees of freedom, exp(-x/2) sum_{i<p} (x/2)^i / i!, which falls strictly in x.
+void joint_thresholds(double amin, double * T)
+{
+    const double q = exp(-0.5 * amin);
+    T[0] = 0.0;
+    T[1] = amin;
+    for (int p = 2; p <= nuslam::kJcbbMMax; ++p)
+    {
+        auto sf = [p](double x) {
+            double t = 1.0, s = 1.0;
+            for (int i = 1; i < p; ++i)
+            {
+                t *= 0.5 * x / i;
+                s += t;
+            }
+            return exp(-0.5 * x) * s;
+        };
+        double lo = T[p - 1], hi = 2.0 * lo + 8.0;
+        while (sf(hi) > q && hi < 1e300) hi *= 2.0;
+        for (int it = 0; it < 2000; ++it)
+        {
+            const double mid = 0.5 * (lo + hi);
+            if (!(mid > lo && mid < hi)) break;
+            if (sf(mid) > q) lo = mid;
+            else hi = mid;
+        }
+        T[p] = hi;
+    }
+}
+
+// NUSLAM_OPT_JOINT_COMPATIBILITY searches at most kJcbbMMax measurements per step (checked before any work of a step is enqueued)
+int joint_m_check(const nuslam_ekf * h, bool unknown_ids, int m)
+{
+    if ((h->cfg.options & NUSLAM_OPT_JOINT_COMPATIBILITY) && unknown_ids && m > nuslam::kJcbbMMax)
+        return fail(NUSLAM_ERR_UNSUPPORTED, "NUSLAM_OPT_JOINT_COMPATIBILITY associates at most 16 measurements per step");
+    return NUSLAM_OK;
 }
 
 template <int OP>
@@ -359,8 +401,14 @@ int nuslam_ekf_create(const nuslam_ekf_config * cfg, int64_t batch, int device, 
     if (!cfg || !out) return fail(NUSLAM_ERR_INVALID, "null config or output pointer");
     if (cfg->n_landmarks < 1 || batch < 1) return fail(NUSLAM_ERR_INVALID, "n_landmarks and batch must be >= 1");
     if (cfg->mode != NUSLAM_MODE_STRICT && cfg->mode != NUSLAM_MODE_FAST && cfg->mode != NUSLAM_MODE_LARGE) return fail(NUSLAM_ERR_INVALID, "unknown mode");
-    if (cfg->options & ~(uint32_t) (NUSLAM_OPT_WRAP_INNOVATION | NUSLAM_OPT_JOSEPH | NUSLAM_OPT_PRE_MOTION_JACOBIAN | NUSLAM_OPT_NEAREST_NEIGHBOUR))
+    if (cfg->options & ~(uint32_t) (NUSLAM_OPT_WRAP_INNOVATION | NUSLAM_OPT_JOSEPH | NUSLAM_OPT_PRE_MOTION_JACOBIAN | NUSLAM_OPT_NEAREST_NEIGHBOUR |
+                                    NUSLAM_OPT_JOINT_COMPATIBILITY))
         return fail(NUSLAM_ERR_INVALID, "unknown option bit");
+    const bool joint = (cfg->options & NUSLAM_OPT_JOINT_COMPATIBILITY) != 0;
+    if (joint && (cfg->options & NUSLAM_OPT_NEAREST_NEIGHBOUR))
+        return fail(NUSLAM_ERR_INVALID, "NUSLAM_OPT_JOINT_COMPATIBILITY and NUSLAM_OPT_NEAREST_NEIGHBOUR exclude each other");
+    if (joint && !(std::isfinite(cfg->assoc_min) && cfg->assoc_min > 0.0))
+        return fail(NUSLAM_ERR_INVALID, "NUSLAM_OPT_JOINT_COMPATIBILITY needs a finite assoc_min > 0 (a chi-square gate at 2 dof)");
     if (!(cfg->landmark_prior > 0.0)) return fail(NUSLAM_ERR_INVALID, "landmark_prior must be positive (default config sets INT_MAX)");
     int ndev = 0;
     cudaError_t e = cudaGetDeviceCount(&ndev);
@@ -378,10 +426,15 @@ int nuslam_ekf_create(const nuslam_ekf_config * cfg, int64_t batch, int device, 
     h->len = 3 + 2 * cfg->n_landmarks;
     h->device = device;
     h->sm_count = prop.multiProcessorCount;
-    h->strict_smem = sizeof(double) * (size_t) nuslam::strict_smem_doubles(h->len);
+    h->strict_smem = sizeof(double) * (size_t) (nuslam::strict_smem_doubles(h->len) + (joint ? nuslam::jcbb_smem_doubles(cfg->n_landmarks) : 0));
     h->strict_warps = 4;
     while (h->strict_warps > 1 && h->strict_smem * h->strict_warps > 200 * 1024) h->strict_warps /= 2;
     if (cfg->mode == NUSLAM_MODE_LARGE || h->strict_smem * h->strict_warps > (size_t) prop.sharedMemPerBlockOptin) h->large = true;
+    if (joint && h->large)
+    {
+        delete h;
+        return fail(NUSLAM_ERR_UNSUPPORTED, "NUSLAM_OPT_JOINT_COMPATIBILITY runs in the on-chip kernels only (not in large-map mode)");
+    }
     // the register kernel covers n_landmarks <= 12; any larger map (that still fits on chip) runs the oracle-order CUDA kernels
     // (same results to the last bit of the reference's arithmetic, lower throughput) -- a FAST request never fails for its size
     if (!h->large && cfg->mode == NUSLAM_MODE_FAST && !nuslam::fast_supported(cfg->n_landmarks)) h->cfg.mode = NUSLAM_MODE_STRICT;
@@ -433,6 +486,18 @@ int nuslam_ekf_create(const nuslam_ekf_config * cfg, int64_t batch, int device, 
     cudaMemsetAsync(h->sigma, 0, sizeof(double) * l * l * batch, h->stream);
     cudaMemsetAsync(h->seen, 0, sizeof(int32_t) * batch, h->stream);
     cudaMemsetAsync(h->status, 0, sizeof(int32_t) * batch, h->stream);
+    if (joint)
+    {
+        double T[nuslam::kJcbbMMax + 1];
+        joint_thresholds(cfg->assoc_min, T);
+        int rc = h->joint_t.reserve(sizeof(T));
+        if (!rc && cudaMemcpy(h->joint_t.p, T, sizeof(T), cudaMemcpyHostToDevice) != cudaSuccess) rc = fail(NUSLAM_ERR_CUDA, "copy of the joint thresholds");
+        if (rc)
+        {
+            nuslam_ekf_destroy(h);
+            return rc;
+        }
+    }
     *out = h;
     return NUSLAM_OK;
 }
@@ -469,6 +534,7 @@ int nuslam_ekf_destroy(nuslam_ekf * h)
     h->lg_ids_slot.release();
     h->lg_assoc_result.release();
     h->lg_nn_slots.release();
+    h->joint_t.release();
     if (h->worklist) cudaFree(h->worklist);
     if (h->wl_count) cudaFree(h->wl_count);
     h->s_tw.release();
@@ -591,6 +657,8 @@ int nuslam_ekf_associate(nuslam_ekf * h, const double * z, int32_t * id_out, int
     }
     else
         p.ids_out = id_out;
+    // one measurement: joint compatibility is nearest neighbour (T[1] = assoc_min, the same distances)
+    if (p.options & NUSLAM_OPT_JOINT_COMPATIBILITY) p.options = (p.options & ~(unsigned) NUSLAM_OPT_JOINT_COMPATIBILITY) | NUSLAM_OPT_NEAREST_NEIGHBOUR;
     rc = h->large ? large_associate(h, p.z, p.ids_out) : launch_strict<nuslam::kOpAssociate>(h, p);
     if (rc) return rc;
     if (mem == NUSLAM_HOST) CU(cudaMemcpyAsync(id_out, p.ids_out, sizeof(int32_t) * h->batch, cudaMemcpyDeviceToHost, h->stream));
@@ -696,6 +764,7 @@ int step_device(nuslam_ekf * h, const nuslam::EkfParams & p)
         if (p.ids && p.ids_out && m > 0) CU(cudaMemcpyAsync(p.ids_out, p.ids, sizeof(int32_t) * h->batch * m, cudaMemcpyDeviceToDevice, h->stream));
         return NUSLAM_OK;
     }
+    if ((h->cfg.options & NUSLAM_OPT_JOINT_COMPATIBILITY) && !p.ids) return launch_strict<nuslam::kOpStepJoint>(h, p);
     if (h->cfg.mode == NUSLAM_MODE_FAST && h->cfg.options == 0 && m <= nuslam::kFastMMax)
         // known correspondence, or on-device association (ids == NULL): the register kernel, then the strict kernel over the
         // filters it handed over (first touches, new landmarks)
@@ -710,6 +779,7 @@ int nuslam_ekf_step(nuslam_ekf * h, const double * twists, const double * z, con
 {
     if (!h || !twists) return fail(NUSLAM_ERR_INVALID, "null handle or twists");
     if (m < 0 || (m > 0 && !z)) return fail(NUSLAM_ERR_INVALID, "m < 0 or null z");
+    if (joint_m_check(h, ids == nullptr, m)) return NUSLAM_ERR_UNSUPPORTED;
     if (select_device(h)) return NUSLAM_ERR_CUDA;
     nuslam::EkfParams p = make_params(h);
     p.m = m;
@@ -738,6 +808,7 @@ int nuslam_ekf_scan_step(nuslam_ekf * h, const double * twists, const float * ra
 {
     if (!h || !twists || !ranges) return fail(NUSLAM_ERR_INVALID, "null handle, twists or ranges");
     if (m < 1) return fail(NUSLAM_ERR_INVALID, "m < 1");
+    if (joint_m_check(h, true, m)) return NUSLAM_ERR_UNSUPPORTED;
     if (select_device(h)) return NUSLAM_ERR_CUDA;
     const size_t B = (size_t) h->batch;
     nuslam::EkfParams p = make_params(h);
@@ -787,6 +858,7 @@ namespace
 int step_async_impl(nuslam_ekf * h, const double * twists, const double * z, const int32_t * ids_host, const int32_t * ids_dev, const void * packed,
                     bool packed_has_ids, int32_t m, double * x_out)
 {
+    if (joint_m_check(h, !ids_host && !ids_dev && !packed_has_ids, m)) return NUSLAM_ERR_UNSUPPORTED;
     if (select_device(h)) return NUSLAM_ERR_CUDA;
     if (!h->s_in)
     {

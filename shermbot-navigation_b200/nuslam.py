@@ -25,6 +25,9 @@ LIB_PATH = Path(_os.environ.get("NUSLAM_B200_LIB", HERE / "libnuslam_b200.so")) 
 NUSLAM_HOST, NUSLAM_DEVICE = 0, 1
 MODE_STRICT, MODE_FAST, MODE_LARGE = 0, 1, 2
 FILTER_MAP_FULL, FILTER_SINGULAR, FILTER_BAD_ID = 1, 2, 4
+# OPT_JOINT_COMPATIBILITY: a step's search hit its budget of joint tests (4 096) and used the best hypothesis so far; informational,
+# it never freezes a filter
+FILTER_ASSOC_TRUNCATED = 8
 ID_EXCEPTION = -1000
 SCAN_UB = -2000
 
@@ -47,6 +50,11 @@ OPT_WRAP_INNOVATION, OPT_JOSEPH, OPT_PRE_MOTION_JACOBIAN = 1, 2, 4   # include/n
 # 60), and otherwise opens a landmark. Combine it with OPT_WRAP_INNOVATION: an unwrapped bearing innovation near +-pi defeats any
 # distance rule.
 OPT_NEAREST_NEIGHBOUR = 8
+# a step's measurements (at most 16 with unknown ids) associated jointly by joint compatibility branch and bound: the largest set of
+# pairings, each landmark used once, whose stacked innovation passes chi2_{2p}^-1(1 - exp(-assoc_min / 2)); assoc_min is the individual
+# chi-square gate at 2 dof (e.g. 9.21), assoc_max the new-landmark threshold. Excludes OPT_NEAREST_NEIGHBOUR, not in large-map mode;
+# include/nuslam_b200.h NUSLAM_OPT_JOINT_COMPATIBILITY has the exact rule.
+OPT_JOINT_COMPATIBILITY = 32
 
 
 class NuslamError(RuntimeError):
@@ -145,7 +153,9 @@ class BatchedExtendedKalman:
     """B independent ``slam_library::ExtendedKalman`` filters on one B200.
 
     ``assoc_min`` / ``assoc_max`` are associateLandmark's thresholds (0.01 / 60 in the reference). Under ``options`` with
-    OPT_NEAREST_NEIGHBOUR, ``assoc_min`` is the gate of the nearest candidate and ``assoc_max`` the new-landmark threshold."""
+    OPT_NEAREST_NEIGHBOUR, ``assoc_min`` is the gate of the nearest candidate and ``assoc_max`` the new-landmark threshold. Under
+    OPT_JOINT_COMPATIBILITY, ``assoc_min`` is the individual chi-square gate (2 dof) that also fixes the joint thresholds, and
+    ``assoc_max`` the new-landmark threshold; steps with unknown ids then take at most 16 measurements."""
 
     def __init__(self, robotState, mapState=None, Q=None, R=None, n_landmarks=None, mode="strict", device=0,
                  stream=None, assoc_min=0.01, assoc_max=60.0, options=0, landmark_prior=None):

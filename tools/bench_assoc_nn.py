@@ -43,13 +43,13 @@ def classify(ids, seen_before):
     return out
 
 
-def quality(filters, steps):
+def quality(filters, steps, rules=RULES):
     import torch
     dev = torch.device("cuda")
     res = {}
     for geometry in ("benign", "adversarial"):
         sc = synth.ekf_scenario(filters, steps, n=12, seed=7, geometry=geometry, shuffle_order=True)
-        for name, (opts, (amin, amax)) in RULES.items():
+        for name, (opts, (amin, amax)) in rules.items():
             eng = nuslam.BatchedExtendedKalman(sc["robot0"], n_landmarks=12, Q=sc["Q"], R=sc["R"], mode="strict", options=opts,
                                                assoc_min=amin, assoc_max=amax, landmark_prior=100.0)
             counts = dict(matched=0, ambiguous=0, new=0, exception=0)
@@ -62,13 +62,15 @@ def quality(filters, steps):
             st = eng.error_stats(truth_pose=pose).cpu().numpy()
             x, s, _, status = eng.get_state()
             nf = max(st[3], 1.0)
-            # the same pose statistics over the filters still running (a filter frozen by MAP_FULL keeps the pose of the scan that froze it)
-            live = status == 0
+            # the same pose statistics over the filters still running (a filter frozen by MAP_FULL or SINGULAR keeps the pose of the scan
+            # that froze it)
+            live = (status & (nuslam.FILTER_MAP_FULL | nuslam.FILTER_SINGULAR)) == 0
             e = x[live, :3] - sc["poses"][steps - 1]
             e[:, 0] = synth.wrap_pi(e[:, 0])
             nees = np.einsum("bi,bi->b", e, np.linalg.solve(s[live][:, :3, :3], e[:, :, None])[:, :, 0])
             res[f"{geometry}/{name}"] = dict(counts, measurements=filters * steps * 12, map_full_filters=int(((status & nuslam.FILTER_MAP_FULL) != 0).sum()),
                                              singular_filters=int(((status & nuslam.FILTER_SINGULAR) != 0).sum()),
+                                             truncated_filters=int(((status & nuslam.FILTER_ASSOC_TRUNCATED) != 0).sum()),
                                              rmse_position_m=float((st[0] / nf) ** 0.5), mean_pose_nees=float(st[2] / nf),
                                              stats_filters=float(st[3]), stats_bad_status=float(st[6]), live_filters=int(live.sum()),
                                              live_rmse_position_m=float(np.sqrt((e[:, 1:] ** 2).sum(axis=1).mean())) if live.any() else None,
@@ -92,7 +94,7 @@ def timed(stream, reset, call, warmup, steps):
     return e0.elapsed_time(e1) / steps
 
 
-def cost_small(B, steps, warmup, rounds, n=12, seen=11, seed=9):
+def cost_small(B, steps, warmup, rounds, n=12, seen=11, seed=9, variants=None):
     """Oracle-order step, 12 landmark slots, unknown ids, on a built map of 11 landmarks (a full map makes the reference's rule throw
     before it looks at a candidate) measured every step: they stand 0.86 m apart on a 1.5 m ring about the driven circle, Sigma small
     and diagonal. Every measurement lies well inside the gate of its own landmark and far beyond the new-landmark
@@ -125,7 +127,7 @@ def cost_small(B, steps, warmup, rounds, n=12, seen=11, seed=9):
     s0 = torch.diag_embed(dg).expand(B, length, length).contiguous()
     seen0 = torch.full((B,), seen, dtype=torch.int32, device=dev)
     status0 = torch.zeros(B, dtype=torch.int32, device=dev)
-    variants = {"wrap": WRAP, "wrap_nn": WRAP | NN}
+    variants = variants or {"wrap": WRAP, "wrap_nn": WRAP | NN}   # the first is the baseline of the ratios
     engs = {name: nuslam.BatchedExtendedKalman(np.zeros((B, 3)), n_landmarks=n, Q=1e-8 * np.eye(3), R=1e-3 * np.eye(2), mode="strict", options=opts,
                                                assoc_min=9.21, assoc_max=60.0, stream=stream.cuda_stream) for name, opts in variants.items()}
     ids = {}
@@ -133,8 +135,9 @@ def cost_small(B, steps, warmup, rounds, n=12, seen=11, seed=9):
         e.set_state(x0, s0, seen0, status0)
         ids[name] = [e.step(tw[t], z[t], None, return_ids=True) for t in range(T)]
         assert int(e.getStatus().max()) == 0
-    same = all(torch.equal(u, v) for u, v in zip(ids["wrap"], ids["wrap_nn"]))
-    matched = int(sum(int((u > 0).sum()) for u in ids["wrap"]))
+    base = next(iter(variants))
+    same = all(torch.equal(u, v) for name in variants for u, v in zip(ids[base], ids[name]))
+    matched = int(sum(int((u > 0).sum()) for u in ids[base]))
     out = {k: [] for k in variants}
     for _ in range(rounds):
         for name, e in engs.items():
@@ -145,7 +148,7 @@ def cost_small(B, steps, warmup, rounds, n=12, seen=11, seed=9):
     return {"filters": B, "landmark_slots": n, "seen": seen, "m": seen, "ids_identical_between_rules": same, "matched": matched,
             "measurements": B * seen * T,
             "ms_per_step": {k: float(np.median(v)) for k, v in out.items()}, "ms_all_rounds": out,
-            "wrap_nn_over_wrap": float(np.median(out["wrap_nn"]) / np.median(out["wrap"]))}
+            **{f"{k}_over_{base}": float(np.median(out[k]) / np.median(out[base])) for k in variants if k != base}}
 
 
 def cost_large(steps, warmup, rounds, m=12, seed=5):
